@@ -79,7 +79,15 @@ def parse():
                          "S < N: N / S replicas of every shard, each group of S ranks serves its own slice of the query batch")
     ap.add_argument("--scans", type=int, default=1024, help="seq: map keyframes (scans)")
     ap.add_argument("--batch", type=int, default=128, help="seq: query scans per call")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (loop results, candidates, and the match / inlier "
+                         "lists of a seeded sample of queries) to DIR/<name>.npy (float64); --impl ours only, the "
+                         "reference arm is a CPU comparison and is not dumped.  seq: that step keeps its results "
+                         "until they are written, so its later batches take fresh buffers")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def plan_layout(rank, world, shards, nkf, nq):
@@ -177,6 +185,59 @@ def result_crc(loops, cands):
     for a in (loops["frame"], loops["score"], cands["frame"], cands["votes"], cands["score"]):
         c = zlib.crc32(np.ascontiguousarray(a).tobytes(), c)
     return c
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+LOOP_FIELDS = ("frame", "ncand", "score")
+DUMP_CAND_FIELDS = ("frame", "votes", "nmatch", "score", "ninlier", "best_hyp", "R", "t")
+LIST_QUERIES, LIST_CANDS, LIST_LIMIT_BYTES = 64, 4, 16 << 20
+
+
+def search_lists(parts, cands):
+    """Match lists (query descriptor, probe ordinal, DB descriptor) and inlier lists of the first LIST_CANDS
+    candidates of a fixed, seeded sample of LIST_QUERIES queries, as a caller fetches them from the results.
+    parts: (first query, SearchResult) pairs, ascending, covering the queries of `cands`.  Only candidates this
+    rank owns carry lists (sharded databases); inlier lists only for verified candidates (score >= 0).
+    Lists stop at LIST_LIMIT_BYTES."""
+    nq = cands.shape[0]
+    pick = np.sort(np.random.default_rng(1).choice(nq, min(nq, LIST_QUERIES), replace=False))
+    key, m, inl, nbytes = [], [], [], 0
+    for q in pick:
+        q0, res = [p for p in parts if p[0] <= q][-1]
+        cq = cands[q]
+        for c in np.nonzero((cq["frame"] >= 0) & (cq["match_off"] >= 0))[0][:LIST_CANDS]:
+            mq, mc, mg = res.matches(q - q0, int(c), int(cq["nmatch"][c]))
+            il = res.inliers(q - q0, int(c), int(cq["ninlier"][c])) if cq["score"][c] >= 0 else np.zeros(0, np.int32)
+            nbytes += 8 * (3 * mq.size + il.size + 4)
+            if nbytes > LIST_LIMIT_BYTES:
+                break
+            key.append((q, c)); m.append(np.stack([mq, mc, mg], 1)); inl.append(il)
+    key = np.array(key, np.int64).reshape(-1, 2)
+    mm = np.concatenate(m) if m else np.zeros((0, 3), np.int64)
+    return {"list_query": key[:, 0], "list_cand": key[:, 1],
+            "list_match_start": np.cumsum([0] + [len(a) for a in m]),       # lists i: [start[i], start[i+1])
+            "match_q": mm[:, 0], "match_cell": mm[:, 1], "match_g": mm[:, 2],
+            "list_inlier_start": np.cumsum([0] + [len(a) for a in inl]),
+            "inlier": np.concatenate(inl) if inl else np.zeros(0, np.int64)}
+
+
+def dump_outputs(out_dir, loops, cands, lists):
+    """What a caller of the search receives -- loop result and candidate list of every query, plus the lists
+    of search_lists() -- as float64 .npy files; integer fields are exact in float64.  Buffer offsets
+    (match_off, inlier_off) are left out: they locate lists inside the library's buffers and are not
+    results.  Above DUMP_LIMIT_BYTES a fixed, seeded sample of the queries is written; query.npy holds the
+    indices of the rows written."""
+    nq, k = cands.shape
+    row_bytes = 8 * (1 + len(LOOP_FIELDS) + k * sum(int(np.prod(cands.dtype[f].shape)) for f in DUMP_CAND_FIELDS))
+    budget = DUMP_LIMIT_BYTES - (64 << 10) - sum(8 * a.size for a in lists.values())   # 64 KB for the .npy headers
+    keep = min(nq, budget // row_bytes)
+    rows = np.arange(nq) if keep == nq else np.sort(np.random.default_rng(0).choice(nq, keep, replace=False))
+    arrays = dict(lists, query=rows)
+    arrays.update({f"loop_{f}": loops[f][rows] for f in LOOP_FIELDS})
+    arrays.update({f"cand_{f}": cands[f][rows] for f in DUMP_CAND_FIELDS})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float64))
 
 
 def per_probe_model_bytes(st):
@@ -372,13 +433,14 @@ class Timer:
             self.dist.barrier()
         self.torch.cuda.synchronize()
 
-    def __call__(self, fn, steps):
+    def __call__(self, fn, steps, last=None):
+        """times `steps` calls; `last`, when given, is called instead of fn in the final step"""
         e0, e1 = self.torch.cuda.Event(enable_timing=True), self.torch.cuda.Event(enable_timing=True)
         keep = []
         self.barrier()
         e0.record(self.stream)
-        for _ in range(steps):
-            keep.append(fn())
+        for i in range(steps):
+            keep.append(last() if last and i == steps - 1 else fn())
         e1.record(self.stream)
         self.barrier()
         ms = e0.elapsed_time(e1)
@@ -389,7 +451,7 @@ class Timer:
         return ms, keep
 
 
-def sweep_entry(torch, dev, cfg_index, nkf, nq, chunk, peak, steps=5, warmup=3):
+def sweep_entry(torch, dev, cfg_index, nkf, nq, chunk, peak, steps, warmup):
     """one point of queries/s vs DB size (single GPU, device-resident queries)"""
     from sgtd_b200 import capi, synth
     cfg = synth.make_config(cfg_index, nkf, nq)
@@ -426,7 +488,7 @@ def sweep_entry(torch, dev, cfg_index, nkf, nq, chunk, peak, steps=5, warmup=3):
     return out
 
 
-def stage1_record(torch, dev, peak, nscans=128, steps=3, warmup=2):
+def stage1_record(torch, dev, peak, steps, warmup, nscans=128):
     """instance extraction (stage 1) on a batch of labelled 64-beam scans of the configs[1]-shaped street
     sequence, scans resident in HBM: scans/s and GB/s on the SURVEY 8d figure of 24 B/point."""
     from sgtd_b200 import capi, synth, synth_seq
@@ -443,12 +505,12 @@ def stage1_record(torch, dev, peak, nscans=128, steps=3, warmup=2):
         return mgr.extract_instances_ptr(pts.data_ptr(), labs.data_ptr(), off)
 
     for _ in range(warmup):
-        nodes, noff, ninst = step()
+        step()
     l0 = mgr.kernel_launches
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        nodes, noff, ninst = step()
     torch.cuda.synchronize()
     ms = (time.perf_counter() - t0) * 1e3 / steps
     npts = int(off[-1])
@@ -516,11 +578,16 @@ def run_ours(args):
     loops_pin = torch.empty(nq * capi.LOOP_DTYPE.itemsize, dtype=torch.uint8).pin_memory()
     cands_pin = torch.empty(nq * k * capi.CAND_DTYPE.itemsize, dtype=torch.uint8).pin_memory()
 
-    def step_device():
+    held = []                                     # --dump-outputs: the search of the last timed step
+
+    def step_device(keep=False):
         qb = mgr.build(q_dev.data_ptr(), qo)
         res = mgr.search(qb)
         out = res.stats()
-        res.free(); qb.free()                     # buffers go back to the handle's pool
+        if keep:
+            held[:] = [res, qb]
+        else:
+            res.free(); qb.free()                 # buffers go back to the handle's pool
         return out
 
     def step_e2e():
@@ -571,8 +638,13 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     l0 = mgr.kernel_launches
-    ms_dev, kept = timer(step_device, args.steps)
+    ms_dev, kept = timer(step_device, args.steps, last=(lambda: step_device(keep=True)) if args.dump_outputs else None)
     launches = mgr.kernel_launches - l0
+    if held:
+        loops_dump, cands_dump = held[0].download()
+        lists_dump = search_lists([(0, held[0])], cands_dump) if rank == 0 else None   # rank 0 serves queries from 0
+        for b in held:
+            b.free()
     # per-kernel numbers from the timed steps themselves (events recorded inside the library)
     vote_ms, stats, stage = [], None, {}
     for st, tm in kept:
@@ -602,7 +674,12 @@ def run_ours(args):
             return np.concatenate([parts[g * S].cpu().numpy() for g in range(R)])
         loops = np.frombuffer(gather(loops).tobytes(), capi.LOOP_DTYPE)
         cands_h = np.frombuffer(gather(cands_h).tobytes(), capi.CAND_DTYPE).reshape(nq_all, k)
+        if args.dump_outputs:
+            loops_dump = np.frombuffer(gather(loops_dump).tobytes(), capi.LOOP_DTYPE)
+            cands_dump = np.frombuffer(gather(cands_dump).tobytes(), capi.CAND_DTYPE).reshape(nq_all, k)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, loops_dump, cands_dump, lists_dump)
 
     if rank == 0:
         peak, peak_src = measured_peak()
@@ -663,13 +740,13 @@ def run_ours(args):
         if world == 1 and not args.no_extras:
             sweep = []
             for (ci, skf, snq) in ((0, 1000, 256), (2, 10000, 256)):
-                sweep.append(sweep_entry(torch, dev, ci, skf, snq, args.chunk, peak))
+                sweep.append(sweep_entry(torch, dev, ci, skf, snq, args.chunk, peak, args.steps, args.warmup))
             sweep.append({"keyframes": nkf, "queries": nq, "db_descriptors": line["config"]["db_descriptors"],
                           "queries_per_s": line["value"], "ms_per_step": line["ms_per_step"], "vote_kernel_ms": vms,
                           "vote_one_pass_gbs": roof.get("achieved"), "vote_one_pass_frac": roof.get("frac"),
                           "stage_ms": line["stage_ms"]})
             line["db_sweep"] = sweep
-            line["stage1"] = stage1_record(torch, dev, peak)
+            line["stage1"] = stage1_record(torch, dev, peak, args.steps, args.warmup)
         if not args.no_cpu_baseline:
             ncores = os.cpu_count() or 1
             v, nk, npick, tb = cpu_port_sample(cfg, args.cpu_keyframes, args.cpu_queries, ncores)
@@ -736,8 +813,9 @@ def run_seq(args):
     out_loops = np.zeros(nq, capi.LOOP_DTYPE)
     out_cands = np.zeros((nq, k), capi.CAND_DTYPE)
     stage = {}
+    held = []                                    # --dump-outputs: (first query, result, batch) of the last timed step
 
-    def step(host):
+    def step(host, keep=False):
         c0 = 0
         for (pts, labs, off, hp, hl) in batches:
             t = [time.perf_counter()]
@@ -753,16 +831,19 @@ def run_seq(args):
             t.append(time.perf_counter())
             n = len(off) - 1
             out_loops[c0:c0 + n] = loops; out_cands[c0:c0 + n] = cands
-            res.free(); qb.free()
+            if keep:
+                held.append((c0, res, qb))
+            else:
+                res.free(); qb.free()
             c0 += n
             for name, a, b_ in (("stage1_ms", 0, 1), ("stage2_ms", 1, 2), ("stage34_ms", 2, 3)):
                 stage[name] = stage.get(name, 0.0) + (t[b_] - t[a]) * 1e3
 
-    def timed(host, steps):
+    def timed(host, steps, keep_last=False):
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        for _ in range(steps):
-            step(host)
+        for i in range(steps):
+            step(host, keep_last and i == steps - 1)
         torch.cuda.synchronize()
         return (time.perf_counter() - t0) * 1e3
 
@@ -772,8 +853,12 @@ def run_seq(args):
     sampler.start()
     stage.clear()
     l0 = mgr.kernel_launches
-    ms_dev = timed(False, args.steps)
+    ms_dev = timed(False, args.steps, keep_last=bool(args.dump_outputs))
     launches = mgr.kernel_launches - l0
+    if args.dump_outputs:                        # step() leaves the last timed step's results in out_*
+        dump_outputs(args.dump_outputs, out_loops, out_cands, search_lists([(c0, res) for c0, res, _ in held], out_cands))
+        for _, res, qb in held:
+            res.free(); qb.free()
     st_dev = {kk: round(vv / args.steps, 2) for kk, vv in stage.items()}
     ms_e2e = timed(True, args.steps)
     clocks = sampler.stop()

@@ -3,8 +3,9 @@ cluster_manager.hpp, compiled unmodified against the stand-in headers of oracle/
 (oracle/Makefile, oracle/ref_wrap.cpp).
 
 TEST INFRASTRUCTURE ONLY: imported by tests/, and by bench.py's cpu_baseline /
---impl reference legs.  Never by sgtd_b200/.  The library is built in the container that
-has /root/reference; the GPU box receives the prebuilt file with the snapshot.
+--impl reference legs.  Never by sgtd_b200/.  The reference's sources are not part of this
+repository: the library is built where SGTD_REFERENCE_DIR names the upstream SGTD package
+directory (the one holding src/STDesc.cpp), or an already built oracle/_ref/ is used.
 """
 import ctypes as C
 import os
@@ -17,19 +18,23 @@ from .orc import CAND_DTYPE, DESC_DTYPE, DEFAULT_CFG, OrcConfig, _p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = os.path.join(_HERE, "_ref", "libsgtd_ref.so")
-REF_SRC = "/root/reference/src/sgtd/src/STDesc.cpp"
+REF_DIR = os.environ.get("SGTD_REFERENCE_DIR", "")
+REF_SRC = os.path.join(REF_DIR, "src", "STDesc.cpp") if REF_DIR else ""
 
 
 def available():
-    """True if the reference build exists (or can be made: the reference tree is present)."""
-    return os.path.exists(_LIB) or os.path.exists(REF_SRC)
+    """True if the reference build exists (or can be made: SGTD_REFERENCE_DIR names the sources).  A
+    SGTD_REFERENCE_DIR without them is an error, not a reason to go without the reference."""
+    if REF_DIR and not os.path.exists(REF_SRC):
+        raise RuntimeError("SGTD_REFERENCE_DIR=%s holds no src/STDesc.cpp" % REF_DIR)
+    return os.path.exists(_LIB) or bool(REF_DIR)
 
 
 def build():
     if os.path.exists(REF_SRC):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "ref"])
+        subprocess.check_call(["make", "-s", "-C", _HERE, "ref", "REF=" + REF_DIR])
     if not os.path.exists(_LIB):
-        raise RuntimeError("oracle/_ref/libsgtd_ref.so is missing and /root/reference is not present to build it")
+        raise RuntimeError("oracle/_ref/libsgtd_ref.so is missing and SGTD_REFERENCE_DIR names no SGTD sources to build it")
     return _LIB
 
 

@@ -22,10 +22,11 @@ def oracle_lib():
 @pytest.fixture(scope="session")
 def reference_lib():
     """oracle/_ref/libsgtd_ref.so: the reference's own STDesc.cpp / cluster_manager.hpp compiled
-    against the oracle/shim stand-in headers.  Built here when /root/reference exists, otherwise the
-    prebuilt file that ships with the snapshot is used; skipped only if neither is there."""
+    against the oracle/shim stand-in headers.  Built from the upstream SGTD sources that
+    SGTD_REFERENCE_DIR names, otherwise an already built library is used; skipped if neither is there,
+    as those sources are not part of this repository."""
     from oracle import ref
     if not ref.available():
-        pytest.skip("oracle/_ref not built and /root/reference absent")
+        pytest.skip("needs the upstream SGTD sources: set SGTD_REFERENCE_DIR, or build oracle/_ref")
     ref.lib()
     return ref

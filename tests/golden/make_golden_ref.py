@@ -1,13 +1,12 @@
 """Golden vectors produced by the REFERENCE's own code -> tests/golden/ref_stage234_small.npz,
 tests/golden/ref_dcvc_small.npz.
 
-The generator is oracle/_ref/libsgtd_ref.so: /root/reference/src/sgtd/src/STDesc.cpp and
+The generator is oracle/_ref/libsgtd_ref.so: the upstream SGTD package's src/STDesc.cpp and
 include/cluster_manager.hpp compiled unmodified (oracle/Makefile target `ref`) against the
-stand-in Eigen/PCL/ROS headers of oracle/shim/.  /root/reference only exists in the build
-container, so the outputs are committed; the oracle (tests/test_oracle*.py, CPU) and the CUDA
-path (tests/test_gpu_*.py) are both checked against them.
+stand-in Eigen/PCL/ROS headers of oracle/shim/.  Those sources are not part of this repository,
+so the outputs are committed; the oracle (tests/test_reference_build.py, CPU) is checked against them.
 
-    python tests/golden/make_golden_ref.py
+    SGTD_REFERENCE_DIR=<upstream>/src/sgtd python tests/golden/make_golden_ref.py
 """
 import hashlib
 import os

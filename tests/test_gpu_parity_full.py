@@ -3,7 +3,8 @@
   * configs[2] (10k keyframes / 256 queries): 16 queries compared IN FULL with the oracle (votes of
     every keyframe, ranking, match lists, inliers, scores, poses);
   * a 2,000-keyframe database compared with the REFERENCE BUILD itself (oracle/_ref: the reference's
-    STDesc.cpp compiled in place; its MAX_FRAME_N = 20000 stack array and ~0.5 KB STDesc bound the size);
+    STDesc.cpp compiled in place; its MAX_FRAME_N = 20000 stack array and ~0.5 KB STDesc bound the size),
+    and an 80-keyframe database compared with the outputs that build stored in tests/golden/;
   * configs[3] (100k keyframes / 1,024 queries, the bench workload): the joins (16-byte float entries --
     the default -- and the experimental 8-byte cell-relative entries with per-lane loads or bulk-async
     staged tiles; all FP32 pre-filter + exact band) and the per-probe streaming kernel (exact FP64 on every entry) must give
@@ -11,6 +12,7 @@
   * configs[4] (dense 2M-point scan, > 500 instances) and 32 scans of the configs[1] sequence: stage 1
     against the literal per-point oracle.
 """
+import hashlib
 import os
 import zlib
 
@@ -80,6 +82,41 @@ def test_2k_keyframes_against_the_reference_build(reference_lib):
         s = r.search()
         exact += compare_query(res, loops, cands, q, s, nf, votes=False, cells=False)
         total += int((s["cands"]["score"] >= 0).sum())
+    assert exact == total
+
+
+def test_reference_golden_reproduced_by_the_cuda_path():
+    """CUDA path vs what the reference's own STDesc.cpp wrote (tests/golden/ref_stage234_small.npz, written by
+    tests/golden/make_golden_ref.py), no oracle in between and no reference sources needed: every database
+    descriptor byte-equal, candidates, match lists, inlier lists and scores equal, poses bit-equal."""
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_stage234_small.npz"))
+    cfg = synth.make_config(int(g["config_index"]), int(g["n_keyframes"]), int(g["n_queries"]))
+    xyz, lab, off = cfg["db"]
+    qx, ql, qo = cfg["queries"]
+    nf, nq = off.shape[0] - 1, qo.shape[0] - 1
+    mgr = capi.STDescManager(device=0)
+    batch = mgr.build(capi.make_nodes(xyz, lab), off, frame_ids=np.arange(nf, dtype=np.uint32))
+    gd, goff = batch.download()
+    assert (np.diff(goff) == g["db_desc_counts"]).all()
+    assert gd[:goff[8]].tobytes() == g["db_descs_head"].tobytes()
+    assert hashlib.sha256(gd.tobytes()).hexdigest() == str(g["db_descs_sha256"])
+    mgr.add(batch)
+    qb = mgr.build(capi.make_nodes(qx, ql), qo)
+    qd, qoff = qb.download()
+    res = mgr.search(qb)
+    loops, cands = res.download()
+    fields = ("frame", "nmatch", "score", "ninlier", "R", "t")
+    exact = total = 0
+    for q in range(nq):
+        assert qd[qoff[q]:qoff[q + 1]].tobytes() == g[f"q{q}_descs"].tobytes()
+        rc = np.zeros(g[f"q{q}_cand_frame"].shape[0], [(f, capi.CAND_DTYPE[f]) for f in fields])
+        for f in fields:
+            rc[f] = g[f"q{q}_cand_{f}"]
+        best = g[f"q{q}_best"]
+        s = dict(n=rc.shape[0], cands=rc, m_q=g[f"q{q}_m_q"], m_g=g[f"q{q}_m_g"], inl=g[f"q{q}_inl"],
+                 best=(int(best[0]), float(best[1])))
+        exact += compare_query(res, loops, cands, q, s, nf, votes=False, cells=False)
+        total += int((rc["score"] >= 0).sum())
     assert exact == total
 
 

@@ -1,7 +1,7 @@
 """CPU tests that PIN THE ORACLE to the reference's own code.
 
-oracle/_ref/libsgtd_ref.so is /root/reference/src/sgtd/src/STDesc.cpp and
-include/cluster_manager.hpp compiled unmodified (oracle/Makefile, target `ref`) against the
+oracle/_ref/libsgtd_ref.so is the upstream SGTD package's src/STDesc.cpp and
+include/cluster_manager.hpp (SGTD_REFERENCE_DIR) compiled unmodified (oracle/Makefile, target `ref`) against the
 stand-in Eigen / PCL / ROS headers of oracle/shim/.  Everything those files compute --
 BuildSingleScanSTD, AddSTDescs, candidate_selector, candidate_verify, triangle_solver,
 SearchLoop, Combinatorial_Binary_Encoding, clusterManager -- is compared here with the oracle
@@ -151,7 +151,7 @@ def test_oracle_dcvc_equals_reference_cluster_manager(oracle_lib, reference_lib)
         assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and a[2:] == b[2:], t
 
 
-# ---- committed reference-produced fixtures (no /root/reference needed) ------------------------------
+# ---- committed reference-produced fixtures (no reference sources needed) ----------------------------
 def test_oracle_reproduces_reference_golden_stage234(oracle_lib):
     g = np.load(os.path.join(GOLDEN, "ref_stage234_small.npz"))
     cfg = synth.make_config(int(g["config_index"]), int(g["n_keyframes"]), int(g["n_queries"]))
