@@ -1742,7 +1742,7 @@ __global__ void __launch_bounds__(kVerifyThreads, kMinBlocks) k_verify(VerifyPar
   __syncthreads();
   if (tid < H) {
     const float tmax = fmaxf(fabsf(s_posef[tid][9]), fmaxf(fabsf(s_posef[tid][10]), fabsf(s_posef[tid][11])));
-    s_posef[tid][12] = fminf(fmaf(4.0e-5f, tmax, 1.0e-4f), 8.0f);
+    s_posef[tid][12] = fmaf(4.0e-5f, tmax, 1.0e-4f);  // not capped: see the margin of the couple
     s_vote[tid] = 0;
   }
   __syncthreads();
@@ -1778,7 +1778,9 @@ __global__ void __launch_bounds__(kVerifyThreads, kMinBlocks) k_verify(VerifyPar
         if (v0) mx = fmaxf(mx, fmaxf(fabsf(a[i]), fabsf(b[i])));
         if (v1) mx = fmaxf(mx, fmaxf(fabsf(a1[i]), fabsf(b1[i])));
       }
-      mgc = fminf(fmaf(4.0e-5f, mx, 1.0e-4f), 8.0f);  // margin of the couple
+      // margin of the couple.  Not capped: past X ~ 2.2e5 the band reaches below 0 and every vertex that is
+      // not clearly outside is decided in FP64 (a cap below the error bound let FP32 decide wrongly there)
+      mgc = fmaf(4.0e-5f, mx, 1.0e-4f);
     }
 #pragma unroll(kMinBlocks == 4 ? 2 : 1)
     for (int h = 0; h < H; ++h) {
