@@ -150,7 +150,7 @@ struct sgtd_options {
   int stats_unique = 0;   // 1: also count the distinct probed buckets / their entries (sgtd_vote_stats B, Eu)
   int join_parts = 0;     // keyframe-range parts per query group of k_vote_join (0/1: none; 2..4)
   int collect_unroll = 0; // hits a thread of k_collect_inv tests per trip (0 / 1: default; 2, 4: experiments)
-  int verify_impl = 0;    // 0: hypothesis loop of k_verify unrolled by 2 at 4 CTAs/SM; 3: not unrolled at 5 CTAs/SM
+  int verify_impl = 0;    // 3: k_verify with a 64-position pair table, so that nearly every candidate runs in chunks
   int join_hint = 0;      // 1: vote REDs carry an L2 evict-last policy
   int join_impl = 1;      // 1 (default): k_vote_join, 16-byte float entries; experimental joins on 8-byte cell-relative
                           // entries (index rebuilt on request): 0 = k_vote_join8 (per-lane loads), 2 = k_vote_run

@@ -223,7 +223,7 @@ __global__ void __launch_bounds__(kVoteThreads) k_vote(VoteParams P) {
 
 // ============================ packed FP32 ===========================================
 // Blackwell's packed FP32 (FFMA2/FADD2/FMUL2: two IEEE single operations per instruction) halves
-// the issue slots of the FP32 pre-filters of k_vote_join and k_verify.  The packed operands are kept
+// the issue slots of the FP32 pre-filters of k_vote_join.  The packed operands are kept
 // as 64-bit registers (inline PTX) so that loop-invariant pairs stay in aligned register pairs.
 typedef unsigned long long f32x2;
 __device__ __forceinline__ f32x2 pack2(float lo, float hi) {
@@ -245,11 +245,6 @@ __device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) {
 __device__ __forceinline__ f32x2 sub2(f32x2 a, f32x2 b) {
   f32x2 d;
   asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
-__device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) {
-  f32x2 d;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
   return d;
 }
 
@@ -1618,17 +1613,22 @@ __device__ void kabsch3(const float *svf, const float *rvf, double *R, double *t
     t[i] = __dadd_rn(dot3s(-R[i * 3], sc[0], -R[i * 3 + 1], sc[1], -R[i * 3 + 2], sc[2]), rc[i]);
 }
 
-// all three vertex residuals < 3.0 m (STDesc.cpp:487-501); sqrt(x) < 3  <=>  x < 9 exactly
+// |R a + t - b| < 3.0 m for one vertex pair (STDesc.cpp:487-501), in the reference's FP64 operation order;
+// sqrt(x) < 3  <=>  x < 9 exactly
+__device__ __forceinline__ bool vertex_inlier(const double *R, const double *t, double px, double py, double pz,
+                                              double bx, double by, double bz) {
+  const double dx = __dsub_rn(__dadd_rn(dot3s(R[0], px, R[1], py, R[2], pz), t[0]), bx);
+  const double dy = __dsub_rn(__dadd_rn(dot3s(R[3], px, R[4], py, R[5], pz), t[1]), by);
+  const double dz = __dsub_rn(__dadd_rn(dot3s(R[6], px, R[7], py, R[8], pz), t[2]), bz);
+  return sqn3(dx, dy, dz) < 9.0;
+}
+
+// all three vertex residuals < 3.0 m
 __device__ __forceinline__ bool pair_inlier(const double *R, const double *t, const float *a, const float *b) {
   bool ok = true;
 #pragma unroll
-  for (int v = 0; v < 3; ++v) {
-    const double px = (double)a[v * 3], py = (double)a[v * 3 + 1], pz = (double)a[v * 3 + 2];
-    const double dx = __dsub_rn(__dadd_rn(dot3s(R[0], px, R[1], py, R[2], pz), t[0]), (double)b[v * 3]);
-    const double dy = __dsub_rn(__dadd_rn(dot3s(R[3], px, R[4], py, R[5], pz), t[1]), (double)b[v * 3 + 1]);
-    const double dz = __dsub_rn(__dadd_rn(dot3s(R[6], px, R[7], py, R[8], pz), t[2]), (double)b[v * 3 + 2]);
-    ok = ok && (sqn3(dx, dy, dz) < 9.0);
-  }
+  for (int v = 0; v < 3; ++v)
+    ok = ok && vertex_inlier(R, t, a[v * 3], a[v * 3 + 1], a[v * 3 + 2], b[v * 3], b[v * 3 + 1], b[v * 3 + 2]);
   return ok;
 }
 
@@ -1639,7 +1639,8 @@ struct VerifyParams {
   const DescVert *dbv;
   const uint32_t *m_q, *m_g;
   int32_t *inl;
-  double *pose;  // kMaxHyp x 12 doubles per candidate: (R row-major, t) of every hypothesis
+  double *pose;     // kMaxHyp x 12 doubles per candidate: (R row-major, t) of every hypothesis
+  int tab_cap;      // positions of k_verify's distinct-pair table in use (power of two <= kPairTab)
 };
 
 __device__ __forceinline__ void load_pair(const VerifyParams &P, int64_t q0, int64_t j, float *a, float *b) {
@@ -1649,46 +1650,12 @@ __device__ __forceinline__ void load_pair(const VerifyParams &P, int64_t q0, int
   b[0] = y.a.x; b[1] = y.a.y; b[2] = y.a.z; b[3] = y.b.x; b[4] = y.b.y; b[5] = y.b.z; b[6] = y.c.x; b[7] = y.c.y; b[8] = y.c.z;
 }
 
-// k_hypotheses solves the 3-point Kabsch of pair h*skip for every hypothesis (H <= 49 per
-// candidate); k_verify then runs one CTA (4 warps) per candidate with the roles transposed:
-// a thread owns a couple of match pairs (registers, fetched once from HBM/L2) and walks the
-// hypotheses with broadcast shared-memory reads -- every lane is busy whatever H is, and
-// there is no barrier inside the scoring loop.  The warp ballots of every (hypothesis, warp
-// tile) are kept in shared memory: votes are their population counts and the inlier list of
-// the winning hypothesis is read back from them, so nothing is evaluated twice.
-//
-// Hypothesis votes use an FP32 pre-filter: the residual of each vertex is first formed
-// in float (FMA).  With |coordinate|, |t| <= X the float residual components are off by
-// at most ~40*eps32*X, so the squared residual is off by < 16*40*eps32*X near the 3 m
-// boundary; outside the band 9 +- margin(X) the float decision equals the reference's
-// FP64 decision, inside it the vertex is re-evaluated exactly in FP64.  Outcomes are
-// therefore identical to pair_inlier() for every pair (checked bit-for-bit by the tests).
-__device__ __forceinline__ bool vertex_inlier_fast(const float *Rf, const float *tf, const double *R, const double *t,
-                                                   float px, float py, float pz, float bx, float by, float bz,
-                                                   float margin) {
-  const float rx = fmaf(Rf[0], px, fmaf(Rf[1], py, fmaf(Rf[2], pz, tf[0]))) - bx;
-  const float ry = fmaf(Rf[3], px, fmaf(Rf[4], py, fmaf(Rf[5], pz, tf[1]))) - by;
-  const float rz = fmaf(Rf[6], px, fmaf(Rf[7], py, fmaf(Rf[8], pz, tf[2]))) - bz;
-  const float d2 = fmaf(rx, rx, fmaf(ry, ry, rz * rz));
-  if (d2 < 9.0f - margin) return true;
-  if (d2 > 9.0f + margin) return false;
-  // ambiguous: exact FP64 evaluation in the reference's operation order
-  const double dx = __dsub_rn(__dadd_rn(dot3s(R[0], (double)px, R[1], (double)py, R[2], (double)pz), t[0]), (double)bx);
-  const double dy = __dsub_rn(__dadd_rn(dot3s(R[3], (double)px, R[4], (double)py, R[5], (double)pz), t[1]), (double)by);
-  const double dz = __dsub_rn(__dadd_rn(dot3s(R[6], (double)px, R[7], (double)py, R[8], (double)pz), t[2]), (double)bz);
-  return sqn3(dx, dy, dz) < 9.0;
-}
-
-// |R p + t - b|^2 of two pairs at once; each half is an IEEE fmaf chain, the same one vertex_inlier_fast() forms
-__device__ __forceinline__ f32x2 resid2_x2(const f32x2 *R2, const f32x2 *t2, f32x2 px, f32x2 py, f32x2 pz, f32x2 bx,
-                                           f32x2 by, f32x2 bz) {
-  const f32x2 rx = sub2(fma2(R2[0], px, fma2(R2[1], py, fma2(R2[2], pz, t2[0]))), bx);
-  const f32x2 ry = sub2(fma2(R2[3], px, fma2(R2[4], py, fma2(R2[5], pz, t2[1]))), by);
-  const f32x2 rz = sub2(fma2(R2[6], px, fma2(R2[7], py, fma2(R2[8], pz, t2[2]))), bz);
-  return fma2(rx, rx, fma2(ry, ry, mul2(rz, rz)));
-}
-constexpr int kMaxHyp = 50;      // hypotheses per candidate (STDesc.cpp:486-489: skip_len = M / 50 + 1 => H <= 49)
-constexpr int kBitWords = 2048;  // (hypothesis, warp tile) outcome words kept in shared memory; beyond it pass 2 re-evaluates
+constexpr int kMaxHyp = 50;             // hypotheses per candidate (STDesc.cpp:486-489: skip_len = M / 50 + 1 => H <= 49)
+constexpr int kPairTab = 1024;          // open-addressing positions of k_verify's distinct-pair table
+constexpr int kPairCap = kPairTab * 3 / 4;  // distinct pairs it holds (load factor <= 3/4)
+constexpr int kChunkMatches = 2048;     // matches whose three pair ids are kept in shared memory at a time
+static_assert(kMaxHyp - 1 <= 64, "the outcomes of a pair are one 64-bit mask over the hypotheses");
+static_assert(kPairCap <= 1024, "a match keeps its three pair ids in 10 bits each");
 
 // One thread per (candidate, hypothesis): the 3-point Kabsch of match pair h * skip
 // (triangle_solver, STDesc.cpp:574-622), all in FP64.  Kept out of k_verify: its long dependent
@@ -1714,14 +1681,52 @@ __global__ void __launch_bounds__(128) k_hypotheses(VerifyParams P, int nslot) {
   for (int i = 0; i < 3; ++i) o[9 + i] = t[i];
 }
 
-template <int kMinBlocks>
-__global__ void __launch_bounds__(kVerifyThreads, kMinBlocks) k_verify(VerifyParams P) {
+__device__ __forceinline__ uint32_t pair_hash(const uint32_t *w) {
+  uint32_t h = 0x811C9DC5u;
+#pragma unroll
+  for (int i = 0; i < 6; ++i) h = (h ^ w[i]) * 0x01000193u;
+  h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
+  return h ? h : 1u;  // 0 marks an empty position
+}
+
+constexpr int kVotePlanes = 5;  // bit-sliced vote counters: a lane adds up to 2^5 - 1 match masks before a flush
+
+// adds a warp's bit-sliced counters (bit h of plane k: 2^k votes of hypothesis h) to the votes
+__device__ __forceinline__ void flush_votes(unsigned long long *cnt, int H, int lane, int *s_vote) {
+  for (int h = 0; h < H; ++h) {
+    int n = 0;
+#pragma unroll
+    for (int k = 0; k < kVotePlanes; ++k) n += (int)((cnt[k] >> h) & 1ull) << k;
+    n = __reduce_add_sync(0xffffffffu, n);
+    if (lane == 0 && n) atomicAdd(&s_vote[h], n);
+  }
+#pragma unroll
+  for (int k = 0; k < kVotePlanes; ++k) cnt[k] = 0ull;
+}
+
+// One CTA (4 warps) per candidate.  The vertex test of candidate_verify depends on one query vertex, one DB
+// vertex and the hypothesis only, and a candidate's matches are triangles over the same ~100 query and ~100
+// keyframe nodes: its ~3 M vertex tests per hypothesis come from a few hundred distinct (query vertex, DB
+// vertex) pairs.  So the kernel
+//   1. maps each vertex slot of each match to a pair id: an open-addressing table in shared memory keyed on
+//      the bits of the six coordinates (equal bits give equal outcomes; the descriptors' label fields play
+//      no part), rounds of up to 128 matches, one per thread;
+//   2. tests every distinct pair against every hypothesis in FP64, in the reference's operation order
+//      (vertex_inlier), and keeps the outcomes as a 64-bit mask per pair;
+//   3. votes: a match is an inlier of h iff bit h of the AND of its three masks is set; each lane adds
+//      the masks of its matches into bit-sliced counters (a ripple-carry add of 64 one-bit counts at once).
+// The table holds kPairCap pairs and the per-match ids kChunkMatches matches; longer or more varied
+// candidates run in chunks (votes add up across chunks, the table starts over when it fills).  A candidate
+// that took one chunk reads its inlier list back from the masks, the others re-test the best hypothesis.
+__global__ void __launch_bounds__(kVerifyThreads, 4) k_verify(VerifyParams P) {
   __shared__ __align__(16) double s_pose[kMaxHyp][12];  // exact (R,t) of every hypothesis
-  __shared__ __align__(16) float s_posef[kMaxHyp][16];  // rounded to float: R0..R8, t0..t2, margin(|t|), pad
-  // s_bits[h * T + w]: ballots of hypothesis h over warp tile w (couples 32w..32w+31): .x pairs 2c, .y pairs 2c+1
-  __shared__ uint2 s_bits[kBitWords];
+  __shared__ uint32_t s_tag[kPairTab];                  // hash of the pair at a position, 0 = empty
+  __shared__ uint16_t s_uid[kPairTab];                  // pair id at a position
+  __shared__ uint32_t s_key[kPairCap][6];               // pair id -> bits of (query vertex xyz, DB vertex xyz)
+  __shared__ unsigned long long s_hm[kPairCap];         // pair id -> bit h: an inlier under hypothesis h
+  __shared__ uint32_t s_ids[kChunkMatches];             // match of the chunk -> its three pair ids
   __shared__ int s_vote[kMaxHyp];
-  __shared__ int s_best, s_cnt[64 * (kVerifyThreads / 32) + 1];
+  __shared__ int s_npair, s_best, s_cnt[64 * (kVerifyThreads / 32) + 1];
   sgtd_candidate *cd = P.cands + blockIdx.x;
   const int64_t moff = cd->match_off;
   const int M = cd->nmatch;
@@ -1731,110 +1736,120 @@ __global__ void __launch_bounds__(kVerifyThreads, kMinBlocks) k_verify(VerifyPar
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int skip = M / 50 + 1;
   const int H = M / skip;
+  const int cap = P.tab_cap, limit = cap * 3 / 4;
+  const int rmax = min(kVerifyThreads, limit / 3);  // matches per round: each adds at most three pairs
   {
     const double *src = P.pose + (size_t)blockIdx.x * kMaxHyp * 12;
-    for (int i = tid; i < H * 12; i += kVerifyThreads) {
-      const double v = src[i];
-      const int hh = i / 12, e = i - hh * 12;
-      s_pose[hh][e] = v; s_posef[hh][e] = (float)v;
+    for (int i = tid; i < H * 12; i += kVerifyThreads) s_pose[i / 12][i % 12] = src[i];
+  }
+  if (tid < kMaxHyp) s_vote[tid] = 0;
+  int np = limit;  // pairs in the table (the same in every thread): "full" clears it for the first chunk
+  int tested = 0, nchunk = 0;
+  unsigned long long cnt[kVotePlanes] = {};  // this lane's votes, bit-sliced
+  int nadd = 0;                              // masks added since the last flush (the same in the whole warp)
+  // the vertices of match ce + tid, the next one this thread maps: loaded a round ahead, so that the
+  // loads (mostly from HBM: a keyframe's descriptors are read once per candidate) overlap the probing
+  float fa[9], fb[9];
+  if (tid < M) load_pair(P, q0, moff + tid, fa, fb);
+  for (int cb = 0; cb < M; ++nchunk) {
+    if (limit - np < 3 * rmax) {  // no room for another round: start the table over
+      for (int i = tid; i < cap; i += kVerifyThreads) s_tag[i] = 0u;
+      if (tid == 0) s_npair = 0;
+      np = tested = 0;
     }
-  }
-  __syncthreads();
-  if (tid < H) {
-    const float tmax = fmaxf(fabsf(s_posef[tid][9]), fmaxf(fabsf(s_posef[tid][10]), fabsf(s_posef[tid][11])));
-    s_posef[tid][12] = fmaf(4.0e-5f, tmax, 1.0e-4f);  // not capped: see the margin of the couple
-    s_vote[tid] = 0;
-  }
-  __syncthreads();
-  // ---- pass 1: votes of every hypothesis
-  const int ncouple = (M + 1) >> 1;
-  const int T = (ncouple + 31) >> 5;        // warp tiles of the candidate
-  const bool keep = H * T <= kBitWords;     // every outcome bit fits in shared memory
-  const int Tc = keep ? T : kBitWords / H;  // warp tiles per chunk (a single chunk when everything fits)
-  for (int tb = 0; tb < T; tb += Tc) {
-  const int te = min(T, tb + Tc);
-  for (int w = tb + wid; w < te; w += kVerifyThreads / 32) {
-    const int c = w * 32 + lane;
-    uint2 *row = s_bits + (w - tb);
-    // coordinate k of pairs 2c (.x) and 2c+1 (.y): a0..a8 = k 0..8, b0..b8 = k 9..17
-    f32x2 K[18];
-    float mgc = 0.f;
-    const f32x2 negzero2 = pack2(-0.f, -0.f);
-    {
-      float a[9], b[9], a1[9], b1[9];
-      const bool v0 = 2 * c < M, v1 = 2 * c + 1 < M;
+    __syncthreads();
+    // ---- 1. pair ids of the chunk's matches
+    int ce = cb;
+    while (ce < M && ce - cb < kChunkMatches && limit - np >= 3 * rmax) {
+      const int r = min(rmax, min(M - ce, cb + kChunkMatches - ce));
+      uint32_t key[3][6], hsh[3];
+      int pos[3], pid[3] = {0, 0, 0}, st[3] = {0, 0, 0};  // st: 0 resolved, 1 probing, 2 same hash seen
+      if (tid < r) {
 #pragma unroll
-      for (int i = 0; i < 9; ++i) { a[i] = 0.f; a1[i] = 0.f; b[i] = b1[i] = __int_as_float(0x7f800000); }
-      // a missing pair sits at infinity: residual +inf, never an inlier, never ambiguous
-      if (v0) load_pair(P, q0, moff + 2 * c, a, b);
-      if (v1) load_pair(P, q0, moff + 2 * c + 1, a1, b1);
-      float mx = 0.f;
+        for (int v = 0; v < 3; ++v) {
 #pragma unroll
-      for (int i = 0; i < 9; ++i) {
-        // "+ (-0)" is the identity on every float; it makes the pair the result of a packed
-        // instruction, which pins it in an aligned register pair for the whole hypothesis loop
-        // (a plain mov.b64 is copy-propagated by ptxas and re-packed in every iteration)
-        K[i] = add2(pack2(a[i], a1[i]), negzero2); K[9 + i] = add2(pack2(b[i], b1[i]), negzero2);
-        if (v0) mx = fmaxf(mx, fmaxf(fabsf(a[i]), fabsf(b[i])));
-        if (v1) mx = fmaxf(mx, fmaxf(fabsf(a1[i]), fabsf(b1[i])));
+          for (int i = 0; i < 3; ++i) { key[v][i] = __float_as_uint(fa[v * 3 + i]); key[v][3 + i] = __float_as_uint(fb[v * 3 + i]); }
+          hsh[v] = pair_hash(key[v]);
+          pos[v] = hsh[v] & (cap - 1);
+          st[v] = 1;
+        }
       }
-      // margin of the couple.  Not capped: past X ~ 2.2e5 the band reaches below 0 and every vertex that is
-      // not clearly outside is decided in FP64 (a cap below the error bound let FP32 decide wrongly there)
-      mgc = fmaf(4.0e-5f, mx, 1.0e-4f);
-    }
-#pragma unroll(kMinBlocks == 4 ? 2 : 1)
-    for (int h = 0; h < H; ++h) {
-      const float4 p0 = *reinterpret_cast<const float4 *>(&s_posef[h][0]), p1 = *reinterpret_cast<const float4 *>(&s_posef[h][4]),
-                   p2 = *reinterpret_cast<const float4 *>(&s_posef[h][8]);
-      const float mt = s_posef[h][12];
-      f32x2 R2[9], t2[3];
-      R2[0] = pack2(p0.x, p0.x); R2[1] = pack2(p0.y, p0.y); R2[2] = pack2(p0.z, p0.z);
-      R2[3] = pack2(p0.w, p0.w); R2[4] = pack2(p1.x, p1.x); R2[5] = pack2(p1.y, p1.y);
-      R2[6] = pack2(p1.z, p1.z); R2[7] = pack2(p1.w, p1.w); R2[8] = pack2(p2.x, p2.x);
-      t2[0] = pack2(p2.y, p2.y); t2[1] = pack2(p2.z, p2.z); t2[2] = pack2(p2.w, p2.w);
-      float2 dA, dB, dC;
-      unpack2(resid2_x2(R2, t2, K[0], K[1], K[2], K[9], K[10], K[11]), dA.x, dA.y);
-      unpack2(resid2_x2(R2, t2, K[3], K[4], K[5], K[12], K[13], K[14]), dB.x, dB.y);
-      unpack2(resid2_x2(R2, t2, K[6], K[7], K[8], K[15], K[16], K[17]), dC.x, dC.y);
-      // margin(X) = 16 * 40 * eps32 * X (+ slack), X = max |coordinate| of the pairs and |t|
-      const float margin = fmaxf(mgc, mt);
-      const float lo = 9.0f - margin, hi = 9.0f + margin;
-      const float m0 = fmaxf(dA.x, fmaxf(dB.x, dC.x)), m1 = fmaxf(dA.y, fmaxf(dB.y, dC.y));
-      bool in0 = m0 < lo, in1 = m1 < lo;  // all three vertices clearly inside: an inlier
-      const bool amb0 = !(in0 || m0 > hi), amb1 = !(in1 || m1 > hi);
-      if (amb0 || amb1) {
-        // some vertex is inside the band (or not comparable): decide that pair exactly
-        const float Rf[9] = {p0.x, p0.y, p0.z, p0.w, p1.x, p1.y, p1.z, p1.w, p2.x};
-        const float tf[3] = {p2.y, p2.z, p2.w};
-        const double *R = &s_pose[h][0], *t = &s_pose[h][9];
-        float u[18], v[18];  // pair 2c, pair 2c+1
+      if (ce + r + tid < M) load_pair(P, q0, moff + ce + r + tid, fa, fb);  // the next round starts at ce + r
+      for (;;) {
+        // claim an empty position or stop at one with the same hash.  A new pair's key is written by the
+        // thread that claimed it, so a same-hash position is compared only after the barrier.
 #pragma unroll
-        for (int i = 0; i < 18; ++i) unpack2(K[i], u[i], v[i]);
-        if (amb0)
-          in0 = vertex_inlier_fast(Rf, tf, R, t, u[0], u[1], u[2], u[9], u[10], u[11], margin) &&
-                vertex_inlier_fast(Rf, tf, R, t, u[3], u[4], u[5], u[12], u[13], u[14], margin) &&
-                vertex_inlier_fast(Rf, tf, R, t, u[6], u[7], u[8], u[15], u[16], u[17], margin);
-        if (amb1)
-          in1 = vertex_inlier_fast(Rf, tf, R, t, v[0], v[1], v[2], v[9], v[10], v[11], margin) &&
-                vertex_inlier_fast(Rf, tf, R, t, v[3], v[4], v[5], v[12], v[13], v[14], margin) &&
-                vertex_inlier_fast(Rf, tf, R, t, v[6], v[7], v[8], v[15], v[16], v[17], margin);
+        for (int v = 0; v < 3; ++v) {
+          while (st[v] == 1) {
+            uint32_t t = s_tag[pos[v]];
+            if (t == 0u) {
+              t = atomicCAS(&s_tag[pos[v]], 0u, hsh[v]);
+              if (t == 0u) {
+                const int u = atomicAdd(&s_npair, 1);
+                s_uid[pos[v]] = (uint16_t)u;
+#pragma unroll
+                for (int i = 0; i < 6; ++i) s_key[u][i] = key[v][i];
+                pid[v] = u; st[v] = 0;
+                break;
+              }
+            }
+            if (t == hsh[v]) st[v] = 2;
+            else pos[v] = (pos[v] + 1) & (cap - 1);
+          }
+        }
+        __syncthreads();
+        bool again = false;
+#pragma unroll
+        for (int v = 0; v < 3; ++v) {
+          if (st[v] == 2) {
+            const int u = s_uid[pos[v]];
+            bool eq = true;
+#pragma unroll
+            for (int i = 0; i < 6; ++i) eq = eq && s_key[u][i] == key[v][i];
+            if (eq) { pid[v] = u; st[v] = 0; }
+            else { pos[v] = (pos[v] + 1) & (cap - 1); st[v] = 1; again = true; }  // a hash collision: probe on
+          }
+        }
+        if (!__syncthreads_or(again)) break;
       }
-      const unsigned bal0 = __ballot_sync(0xffffffffu, in0), bal1 = __ballot_sync(0xffffffffu, in1);
-      if (lane == 0) *row = make_uint2(bal0, bal1);
-      row += Tc;
+      if (tid < r) s_ids[ce - cb + tid] = (uint32_t)pid[0] | (uint32_t)pid[1] << 10 | (uint32_t)pid[2] << 20;
+      np = s_npair;
+      ce += r;
+      __syncthreads();  // every thread has read s_npair before the next round adds to it
     }
+    // ---- 2. outcomes of the pairs new to the table under every hypothesis
+    for (int u = tested + tid; u < np; u += kVerifyThreads) {
+      const double px = __uint_as_float(s_key[u][0]), py = __uint_as_float(s_key[u][1]), pz = __uint_as_float(s_key[u][2]);
+      const double bx = __uint_as_float(s_key[u][3]), by = __uint_as_float(s_key[u][4]), bz = __uint_as_float(s_key[u][5]);
+      unsigned long long m = 0ull;
+#pragma unroll 2
+      for (int h = 0; h < H; ++h) {
+        const double2 *ps = reinterpret_cast<const double2 *>(&s_pose[h][0]);  // broadcast 16-byte reads
+        double R[12];
+#pragma unroll
+        for (int i = 0; i < 6; ++i) { const double2 x = ps[i]; R[2 * i] = x.x; R[2 * i + 1] = x.y; }
+        if (vertex_inlier(R, R + 9, px, py, pz, bx, by, bz)) m |= 1ull << h;
+      }
+      s_hm[u] = m;
+    }
+    tested = np;
+    __syncthreads();
+    // ---- 3. votes of the chunk's matches
+    const int nc = ce - cb;
+    for (int base = wid * 32; base < nc; base += kVerifyThreads) {
+      const int i = base + lane;
+      unsigned long long m = 0ull;
+      if (i < nc) {
+        const uint32_t w = s_ids[i];
+        m = s_hm[w & 1023u] & s_hm[(w >> 10) & 1023u] & s_hm[w >> 20];
+      }
+#pragma unroll
+      for (int k = 0; k < kVotePlanes; ++k) { const unsigned long long c = cnt[k] & m; cnt[k] ^= m; m = c; }
+      if (++nadd == (1 << kVotePlanes) - 1) { flush_votes(cnt, H, lane, s_vote); nadd = 0; }
+    }
+    cb = ce;
   }
-  __syncthreads();
-  // votes of the chunk: population counts of the ballot words
-  const int nw = te - tb;
-  for (int idx = tid; idx < H * nw; idx += kVerifyThreads) {
-    const int hh = idx / nw;
-    const uint2 bw = s_bits[hh * Tc + (idx - hh * nw)];
-    const int n = __popc(bw.x) + __popc(bw.y);
-    if (n) atomicAdd(&s_vote[hh], n);
-  }
-  if (te < T) __syncthreads();  // the next chunk overwrites the words
-  }
+  flush_votes(cnt, H, lane, s_vote);
   __syncthreads();
   if (tid == 0) {
     int best = 0, mv = 0;
@@ -1844,14 +1859,15 @@ __global__ void __launch_bounds__(kVerifyThreads, kMinBlocks) k_verify(VerifyPar
   __syncthreads();
   const int best = s_best;
   if (best < 0) { if (tid == 0) { cd->score = -1; cd->best_hyp = -1; cd->ninlier = 0; } return; }
+  const bool keep = nchunk == 1;  // every match's pair ids are still in shared memory
   double Rb[9], tb[3];
 #pragma unroll
   for (int i = 0; i < 9; ++i) Rb[i] = s_pose[best][i];
 #pragma unroll
   for (int i = 0; i < 3; ++i) tb[i] = s_pose[best][9 + i];
   // ---- pass 2: inlier list of the best hypothesis, in match order.  Chunks of 64 tiles: the
-  // outcomes (kept ballot bit, or a re-evaluation when they did not fit) go to a per-thread bit mask with no
-  // barrier in between; one scan of the per-(tile, warp) counts gives every inlier its position.
+  // outcomes (from the pair masks, or a re-test when the candidate took several chunks) go to a per-thread
+  // bit mask with no barrier in between; one scan of the per-(tile, warp) counts gives every inlier its position.
   constexpr int kWarps = kVerifyThreads / 32;
   int ninl = 0;
   for (int cb = 0; cb < M; cb += 64 * kVerifyThreads) {
@@ -1862,8 +1878,8 @@ __global__ void __launch_bounds__(kVerifyThreads, kMinBlocks) k_verify(VerifyPar
       bool ok = false;
       if (j < M) {
         if (keep) {
-          const uint2 w = s_bits[best * T + (j >> 6)];
-          ok = (((j & 1) ? w.y : w.x) >> ((j >> 1) & 31)) & 1u;
+          const uint32_t w = s_ids[j];
+          ok = ((s_hm[w & 1023u] & s_hm[(w >> 10) & 1023u] & s_hm[w >> 20]) >> best) & 1ull;
         } else {
           float a[9], b[9];
           load_pair(P, q0, moff + j, a, b);
@@ -2266,10 +2282,12 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r) {
     W.m_q = r->m_q.p; W.m_g = r->m_g.p; W.inl = r->inl.p; W.pose = (double *)(S + o_pose);
     k_hypotheses<<<(unsigned)(((size_t)nslot * kMaxHyp + 127) / 128), 128, 0, st>>>(W, (int)nslot);
     SGTD_LAUNCHED(h);
-    // default: hypothesis loop unrolled by 2 at 4 CTAs/SM (measured 9.00 ms on the bench workload; not unrolled at
-    // 5 CTAs/SM -- option verify_impl = 3 -- 9.26; at 6 CTAs/SM with 80 registers 9.54; unrolled by 4 at 3 CTAs/SM 8.97)
-    if (h->opt.verify_impl == 3) k_verify<5><<<(unsigned)nslot, kVerifyThreads, 0, st>>>(W);
-    else k_verify<4><<<(unsigned)nslot, kVerifyThreads, 0, st>>>(W);
+    // k_verify tests each distinct (query vertex, DB vertex) pair of a candidate once per hypothesis, in FP64.
+    // Option verify_impl = 3 shrinks its pair table to 64 positions (48 pairs), so that nearly every candidate
+    // runs in chunks and re-tests its best hypothesis for the inlier list: the same results through the
+    // overflow path.
+    W.tab_cap = h->opt.verify_impl == 3 ? 64 : kPairTab;
+    k_verify<<<(unsigned)nslot, kVerifyThreads, 0, st>>>(W);
     SGTD_LAUNCHED(h);
     SGTD_CUDA(h, cudaGetLastError());
   }
