@@ -174,7 +174,7 @@ int64_t sgtd_kernel_launches(const sgtd_handle *h);   /* kernels launched so far
  * "join_impl" (1 default; 0 / 2 experimental joins on 8-byte entries), "join_parts" (2..4: keyframe-range
  * passes inside a query group), "join_hint" (vote REDs with an L2 evict-last policy), "collect_unroll",
  * "verify_impl", "stats_unique", "s1_trace", "s1_replay" (1 = sequential stage-1 replay forms only; default 0 =
- * component-parallel replay), "s1_rows", "s1_table";
+ * component-parallel replay), "s1_rows", "s1_table", "gicp_wave", "gicp_cell_um" (see sgtd_gicp_map_add);
  * "s1_variant" (1 = class tables of local_map_creation) is the one that selects behaviour.  The same
  * switches are read once from the environment by sgtd_create (SGTD_VOTE_MODE=stream, SGTD_JOIN_GROUPS,
  * SGTD_COLLECT_MODE=desc|inv, SGTD_COLLECT_GROUP, SGTD_DEBUG_NOVOTE); sgtd_search never reads the
@@ -365,7 +365,9 @@ int sgtd_gicp_params_default(sgtd_gicp_params *p);
  * distribution-to-distribution cost.  final12 = reg.getFinalTransformation() (3x4, the values of the float
  * matrix), *fitness = reg.getFitnessScore() (mean squared nearest-neighbour distance of the aligned source).
  * Clouds may be host or device memory.  Floating point: agrees with the CPU restatement within
- * 1e-6 (transform) / 1e-6 relative (fitness), see tests/test_gpu_gicp.py. */
+ * 1e-5 (transform) / 1e-5 relative (fitness), see tests/test_gicp.py.  The target is uploaded as a
+ * transient cloud (covariances + nearest-neighbour grid), kept while params->reuse_target is set and the
+ * same buffer is passed again. */
 int sgtd_gicp_align(sgtd_handle *h, const float *source_xyz, int64_t n_source, const float *target_xyz,
                     int64_t n_target, const double *init12, const sgtd_gicp_params *params,
                     double *final12, double *fitness, int32_t *iterations, int32_t *converged);
@@ -379,6 +381,38 @@ int sgtd_gicp_refine_candidates(sgtd_handle *h, const float *source_xyz, int64_t
                                 const sgtd_candidate *cands, const int32_t *order, int32_t ncand,
                                 const sgtd_gicp_params *params, int32_t *chosen, double *transformation12,
                                 double *fitness, int32_t *n_aligned);
+
+/* Keyframe clouds for GICP targets (the map keyframes' clouds, R/src/semantic_graph_localization.cpp:651-721),
+ * held on the handle's device and keyed by global keyframe id (independent of sharding).  Cloud s is
+ * xyz[offsets[s] .. offsets[s+1]) (n x 3 floats, host or device; offsets, frame_ids host); frame_ids NULL =
+ * consecutive from sgtd_gicp_map_frames(h).  Per-point covariances (params->num_neighbors, PLANE) and the
+ * nearest-neighbour grid are built here, once.  A frame id added twice, a cloud with fewer than
+ * num_neighbors points, or a num_neighbors different from the clouds already held: SGTD_E_INVALID.
+ * The grid's cell size is automatic (about one cell per point over the cloud's bounding box) unless
+ * option "gicp_cell_um" is set; it changes speed only, never a result. */
+int sgtd_gicp_map_add(sgtd_handle *h, const float *xyz, const int64_t *offsets, int32_t nclouds,
+                      const uint32_t *frame_ids, const sgtd_gicp_params *params);
+int64_t sgtd_gicp_map_frames(const sgtd_handle *h); /* clouds held */
+int sgtd_gicp_map_clear(sgtd_handle *h);
+/* Exact nearest stored point (index within that keyframe's cloud, squared float distance in FLANN's
+ * L2_Simple order; ties to the lower index) of n query points.  xyz, idx, sqdist: host or device. */
+int sgtd_gicp_map_nearest(sgtd_handle *h, uint32_t frame, const float *xyz, int64_t n, int32_t *idx,
+                          float *sqdist);
+/* The node's multi-candidate loop (sgtd_gicp_refine_candidates) for nq queries at once.  Source of query q:
+ * sources_xyz[src_offsets[q] .. src_offsets[q+1]) (host or device).  Candidates of q:
+ * cands[q*cand_stride .. + ncand[q]), visited in order[q*cand_stride + i] (NULL = as given); the target is
+ * the stored cloud of cand.frame; a candidate with frame < 0 or without a stored cloud is skipped.
+ * src_offsets, cands, ncand, order and the outputs are host arrays; outputs per query as in
+ * sgtd_gicp_refine_candidates (transformation12: 12 doubles per query), bit for bit.  Candidates are
+ * aligned in waves (option "gicp_wave": candidates per query and wave, 0 = automatic); results after a
+ * query's stopping point are discarded, so no output depends on the wave size. */
+int sgtd_gicp_refine_batch(sgtd_handle *h, const float *sources_xyz, const int64_t *src_offsets, int32_t nq,
+                           const sgtd_candidate *cands, int32_t cand_stride, const int32_t *ncand,
+                           const int32_t *order, const sgtd_gicp_params *params, int32_t *chosen,
+                           double *transformation12, double *fitness, int32_t *n_aligned);
+/* Work of the last sgtd_gicp_refine_batch / sgtd_gicp_refine_candidates / sgtd_gicp_align call: problems
+ * aligned (source, candidate pairs), waves, and rounds (one batched evaluation + one copy to the host each). */
+int sgtd_gicp_refine_stats(const sgtd_handle *h, int64_t *problems, int32_t *waves, int32_t *rounds);
 
 #ifdef __cplusplus
 }

@@ -106,6 +106,12 @@ SYMBOLS = {
     "sgtd_gicp_params_default": (C.c_int, [C.POINTER(GicpParams)]),
     "sgtd_gicp_align": (C.c_int, [_VP, _VP, _I64, _VP, _I64, _VP, C.POINTER(GicpParams), _VP, _VP, _VP, _VP]),
     "sgtd_gicp_refine_candidates": (C.c_int, [_VP, _VP, _I64, _VP, _VP, _VP, _VP, _I32, C.POINTER(GicpParams), _VP, _VP, _VP, _VP]),
+    "sgtd_gicp_map_add": (C.c_int, [_VP, _VP, _VP, _I32, _VP, C.POINTER(GicpParams)]),
+    "sgtd_gicp_map_frames": (_I64, [_VP]),
+    "sgtd_gicp_map_clear": (C.c_int, [_VP]),
+    "sgtd_gicp_map_nearest": (C.c_int, [_VP, _U32, _VP, _I64, _VP, _VP]),
+    "sgtd_gicp_refine_batch": (C.c_int, [_VP, _VP, _VP, _I32, _VP, _I32, _VP, _VP, C.POINTER(GicpParams), _VP, _VP, _VP, _VP]),
+    "sgtd_gicp_refine_stats": (C.c_int, [_VP, C.POINTER(_I64), C.POINTER(_I32), C.POINTER(_I32)]),
     "sgtd_set_option": (C.c_int, [_VP, C.c_char_p, C.c_int32]),
     "sgtd_recall_rank": (C.c_int, [_VP, C.c_int32, _VP, C.c_int64, _VP, C.c_double, _VP, _VP]),
 }
@@ -356,6 +362,60 @@ class STDescManager:
         self._chk(lib().sgtd_gicp_refine_candidates(self._h, _p(source), source.shape[0], ptrs, _p(sizes), _p(cands), _p(order), n,
                                                     C.byref(p), C.byref(chosen), _p(T), C.byref(fit), C.byref(nal)))
         return chosen.value, T.reshape(3, 4), fit.value, nal.value
+
+    # -- keyframe cloud store + batched refinement --------------------------------------------------
+    def gicp_map_add(self, xyz, offsets=None, frame_ids=None, params=None):
+        """Store keyframe clouds (n x 3 float32 host array, or a raw device pointer with offsets)."""
+        if isinstance(xyz, np.ndarray):
+            xyz = np.ascontiguousarray(xyz, np.float32).reshape(-1, 3)
+            if offsets is None:
+                offsets = np.array([0, xyz.shape[0]], np.int64)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        ids = None if frame_ids is None else np.ascontiguousarray(frame_ids, np.uint32)
+        p = params or self.gicp_params()
+        self._chk(lib().sgtd_gicp_map_add(self._h, _p(xyz), _p(offsets), offsets.shape[0] - 1, _p(ids), C.byref(p)))
+
+    def gicp_map_frames(self):
+        return int(lib().sgtd_gicp_map_frames(self._h))
+
+    def gicp_map_clear(self):
+        self._chk(lib().sgtd_gicp_map_clear(self._h))
+
+    def gicp_map_nearest(self, frame, xyz, n=None):
+        """-> (index within the stored cloud int32 [n], squared float distance float32 [n])"""
+        if isinstance(xyz, np.ndarray):
+            xyz = np.ascontiguousarray(xyz, np.float32).reshape(-1, 3)
+            n = xyz.shape[0]
+        idx = np.zeros(max(n, 1), np.int32)
+        d = np.zeros(max(n, 1), np.float32)
+        self._chk(lib().sgtd_gicp_map_nearest(self._h, int(frame), _p(xyz), n, _p(idx), _p(d)))
+        return idx[:n], d[:n]
+
+    def gicp_refine_batch(self, sources, src_offsets, cands, ncand, order=None, params=None):
+        """The node's candidate loop for every query against the stored clouds.  sources: n x 3 float32
+        (host array or raw device pointer), cands: CAND_DTYPE [nq, stride], ncand int32 [nq], order int32
+        [nq, stride] or None -> (chosen int32 [nq], transformation [nq, 3, 4], fitness [nq], n_aligned [nq])"""
+        if isinstance(sources, np.ndarray):
+            sources = np.ascontiguousarray(sources, np.float32).reshape(-1, 3)
+        src_offsets = np.ascontiguousarray(src_offsets, np.int64)
+        nq = src_offsets.shape[0] - 1
+        cands = np.ascontiguousarray(cands, CAND_DTYPE).reshape(nq, -1)
+        ncand = np.ascontiguousarray(ncand, np.int32)
+        order = None if order is None else np.ascontiguousarray(order, np.int32).reshape(nq, cands.shape[1])
+        p = params or self.gicp_params()
+        chosen = np.zeros(max(nq, 1), np.int32)
+        T = np.zeros((max(nq, 1), 12))
+        fit = np.zeros(max(nq, 1))
+        nal = np.zeros(max(nq, 1), np.int32)
+        self._chk(lib().sgtd_gicp_refine_batch(self._h, _p(sources), _p(src_offsets), nq, _p(cands), cands.shape[1], _p(ncand),
+                                               _p(order), C.byref(p), _p(chosen), _p(T), _p(fit), _p(nal)))
+        return chosen[:nq], T[:nq].reshape(nq, 3, 4), fit[:nq], nal[:nq]
+
+    def gicp_refine_stats(self):
+        """(problems, waves, rounds) of the last refinement call"""
+        pb, w, r = C.c_int64(0), C.c_int32(0), C.c_int32(0)
+        self._chk(lib().sgtd_gicp_refine_stats(self._h, C.byref(pb), C.byref(w), C.byref(r)))
+        return pb.value, w.value, r.value
 
     def set_option(self, name, value):
         """experiment / parity switches (sgtd_set_option): vote_stream, join_groups, collect_mode, ..."""

@@ -248,6 +248,8 @@ int sgtd_set_option(sgtd_handle *h, const char *name, int32_t value) {
   else if (!strcmp(name, "s1_rows")) h->opt.s1_rows = value != 0;
   else if (!strcmp(name, "s1_replay")) h->opt.s1_replay = value == 1;
   else if (!strcmp(name, "s1_table")) h->opt.s1_table = value == 1;
+  else if (!strcmp(name, "gicp_wave")) h->opt.gicp_wave = std::max(0, (int)value);
+  else if (!strcmp(name, "gicp_cell_um")) h->opt.gicp_cell_um = std::max(0, (int)value);
   else SGTD_FAIL(h, SGTD_E_INVALID, "unknown option");
   return SGTD_OK;
 }

@@ -155,6 +155,8 @@ struct sgtd_options {
   int join_impl = 1;      // 1 (default): k_vote_join, 16-byte float entries; experimental joins on 8-byte cell-relative
                           // entries (index rebuilt on request): 0 = k_vote_join8 (per-lane loads), 2 = k_vote_run
                           // (bulk-async staged tiles).  Measured on the bench workload: 9.0 / 11.4 / 12.6 ms.
+  int gicp_wave = 0;      // candidates per query and GICP wave (0: automatic, 1, 2, 4, ... per wave)
+  int gicp_cell_um = 0;   // cell size of the nearest-neighbour grids built from now on, micrometres (0: automatic)
 };
 
 struct sgtd_handle {
