@@ -389,7 +389,10 @@ int sgtd_gicp_refine_candidates(sgtd_handle *h, const float *source_xyz, int64_t
  * nearest-neighbour grid are built here, once.  A frame id added twice, a cloud with fewer than
  * num_neighbors points, or a num_neighbors different from the clouds already held: SGTD_E_INVALID.
  * The grid's cell size is automatic (about one cell per point over the cloud's bounding box) unless
- * option "gicp_cell_um" is set; it changes speed only, never a result. */
+ * option "gicp_cell_um" is set; it changes speed only, never a result.  On a handle sharded with a
+ * communicator (sgtd_shard_init with nranks > 1 and an NCCL id), give each rank the clouds of its own
+ * keyframe range: sgtd_gicp_refine_batch looks a frame up only on the rank that owns it and ignores the
+ * other clouds a rank holds.  The store itself keeps whatever it is given. */
 int sgtd_gicp_map_add(sgtd_handle *h, const float *xyz, const int64_t *offsets, int32_t nclouds,
                       const uint32_t *frame_ids, const sgtd_gicp_params *params);
 int64_t sgtd_gicp_map_frames(const sgtd_handle *h); /* clouds held */
@@ -405,13 +408,26 @@ int sgtd_gicp_map_nearest(sgtd_handle *h, uint32_t frame, const float *xyz, int6
  * src_offsets, cands, ncand, order and the outputs are host arrays; outputs per query as in
  * sgtd_gicp_refine_candidates (transformation12: 12 doubles per query), bit for bit.  Candidates are
  * aligned in waves (option "gicp_wave": candidates per query and wave, 0 = automatic); results after a
- * query's stopping point are discarded, so no output depends on the wave size. */
+ * query's stopping point are discarded, so no output depends on the wave size.
+ * On a handle sharded with a communicator (sgtd_shard_init with nranks > 1 and an NCCL id) the call is
+ * collective, like sgtd_search: every rank of the group calls it with the same arguments (and the same
+ * "gicp_wave"), e.g. the candidates sgtd_search merged.  Candidate (q, i) belongs to the rank whose
+ * sgtd_shard_init keyframe range holds cand.frame (the last range is open-ended); only that rank looks the
+ * frame up in its store and aligns it.  One all-reduce of a word per candidate slot tells every rank which
+ * candidates are held and whether the call fails (SGTD_E_INVALID on every rank alike, before any
+ * alignment); after each wave one all-reduce hands every rank the wave's results.  Every rank returns the
+ * same outputs, bit for bit those of an unsharded handle holding the union of what each owner holds for
+ * its own range.  Handles without a communicator (unsharded, or virtual shards with a NULL id) look up
+ * every candidate in their own store. */
 int sgtd_gicp_refine_batch(sgtd_handle *h, const float *sources_xyz, const int64_t *src_offsets, int32_t nq,
                            const sgtd_candidate *cands, int32_t cand_stride, const int32_t *ncand,
                            const int32_t *order, const sgtd_gicp_params *params, int32_t *chosen,
                            double *transformation12, double *fitness, int32_t *n_aligned);
 /* Work of the last sgtd_gicp_refine_batch / sgtd_gicp_refine_candidates / sgtd_gicp_align call: problems
- * aligned (source, candidate pairs), waves, and rounds (one batched evaluation + one copy to the host each). */
+ * aligned (source, candidate pairs), waves, and rounds (one batched evaluation + one copy to the host each).
+ * After a sharded sgtd_gicp_refine_batch (a handle with a communicator), problems and rounds are this rank's
+ * own (the problems summed over the ranks are the unsharded call's); waves is the whole call's, the same
+ * on every rank and equal to the unsharded call's. */
 int sgtd_gicp_refine_stats(const sgtd_handle *h, int64_t *problems, int32_t *waves, int32_t *rounds);
 
 #ifdef __cplusplus

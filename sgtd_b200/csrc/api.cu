@@ -410,7 +410,7 @@ int sgtd_add_descriptors(sgtd_handle *h, const sgtd_desc_batch *b) {
   // range of scans this rank owns
   int s0 = 0, s1 = b->nscans;
   if (h->frames_per_rank > 0) {
-    const int64_t lo = h->frame_lo(), hi = (h->rank == h->nranks - 1) ? (1ll << 40) : lo + h->frames_per_rank;
+    const int64_t lo = h->frame_lo(), hi = h->frame_hi();
     s0 = (int)std::min<int64_t>(std::max<int64_t>(lo - (int64_t)first, 0), b->nscans);
     s1 = (int)std::min<int64_t>(std::max<int64_t>(hi - (int64_t)first, 0), b->nscans);
     if ((int64_t)first + s0 != h->frame_lo() + h->frames_local() && s1 > s0)

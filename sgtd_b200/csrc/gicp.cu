@@ -25,6 +25,7 @@
 #include <cub/device/device_segmented_radix_sort.cuh>
 
 #include "internal.cuh"
+#include "nccl_dyn.h"
 #include "svd3.cuh"
 
 namespace sgtd {
@@ -597,13 +598,14 @@ struct GicpPool {
   DevBuf<float> sqd;
   DevBuf<GicpProb> prob;
   DevBuf<int64_t> soff;
+  DevBuf<uint32_t> xw;  // words of a sharded call's all-reduces
   // counters of the last refine call
   int64_t st_problems = 0;
   int32_t st_waves = 0, st_rounds = 0;
   ~GicpPool() {
     in_xyz.release(); key0.release(); key1.release(); val0.release(); val1.release(); flag.release(); cid.release();
     segoff.release(); off.release(); cub.release(); in_s.release(); src.release(); cov_s.release(); mahal.release();
-    partial.release(); out.release(); corr.release(); sqd.release(); prob.release(); soff.release();
+    partial.release(); out.release(); corr.release(); sqd.release(); prob.release(); soff.release(); xw.release();
   }
 };
 static void gicp_pool_free(void *p) { delete static_cast<GicpPool *>(p); }
@@ -800,12 +802,15 @@ struct Visit { int32_t c; const GicpCloud *tgt; const sgtd_candidate *cd; };
 struct QueryIn { const float *xyz; int32_t ns; std::vector<Visit> visit; };
 // sets ProbIn::tgt of a wave's problems whose Visit has none (targets prepared per wave)
 using ResolveTargets = std::function<int(std::vector<ProbIn> &, const std::vector<const Visit *> &)>;
+// aligns a wave's problems (replaces solve_problems, e.g. for a sharded call)
+using SolveWave = std::function<int(const std::vector<ProbIn> &, std::vector<ProbOut> &)>;
 
 // The node's candidate loop for every query, in waves: each wave aligns the next W unvisited candidates of
 // every unfinished query, then applies the sequential rule in visit order (lowest fitness below 100 wins,
 // the first below best_fitness ends the search; later results of that query are discarded).
 static int refine_queries(sgtd_handle *h, GicpPool &P, const std::vector<QueryIn> &Q, int k, const sgtd_gicp_params &prm,
-                          int32_t *chosen, double *T12, double *fit, int32_t *nal, const ResolveTargets &resolve = nullptr) {
+                          int32_t *chosen, double *T12, double *fit, int32_t *nal, const ResolveTargets &resolve = nullptr,
+                          const SolveWave &solve = nullptr) {
   const double I12[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
   const size_t nq = Q.size();
   std::vector<size_t> pos(nq, 0);
@@ -841,7 +846,7 @@ static int refine_queries(sgtd_handle *h, GicpPool &P, const std::vector<QueryIn
     ++P.st_waves;
     if (resolve)
       if (int rc = resolve(in, vis)) return rc;
-    if (int rc = solve_problems(h, P, in, k, prm, out)) return rc;
+    if (int rc = solve ? solve(in, out) : solve_problems(h, P, in, k, prm, out)) return rc;
     for (size_t i = 0; i < in.size(); ++i) {
       const size_t q = who[i].first;
       if (done[q]) continue;  // past this query's stopping point
@@ -853,6 +858,49 @@ static int refine_queries(sgtd_handle *h, GicpPool &P, const std::vector<QueryIn
     }
     for (size_t q = 0; q < nq; ++q)
       if (!done[q]) { pos[q] += W; if (pos[q] >= Q[q].visit.size()) done[q] = 1; }
+  }
+  return SGTD_OK;
+}
+
+// ---- sharded refinement (a handle with a communicator) ------------------------------------------------------
+// Sum all-reduce of w over the handle's communicator, staged through a device buffer.  Every word has one
+// writer and zeros on the other ranks, so the sums are the writers' words (bit patterns of doubles included).
+static int allreduce_words(sgtd_handle *h, GicpPool &P, std::vector<uint32_t> &w) {
+  if (w.empty()) return SGTD_OK;
+  const cudaStream_t st = h->stream;
+  G_CUDA(P.xw.reserve(w.size(), st, false));
+  G_CUDA(cudaMemcpyAsync(P.xw.p, w.data(), w.size() * 4, cudaMemcpyHostToDevice, st));
+  if (nccl_api().AllReduce(P.xw.p, P.xw.p, w.size(), ncclUint32, ncclSum, (ncclComm_t)h->nccl, st) != ncclSuccess)
+    return sgtd_fail(h, SGTD_E_NCCL, "ncclAllReduce(gicp)", __FILE__, __LINE__);
+  G_CUDA(cudaMemcpyAsync(w.data(), P.xw.p, w.size() * 4, cudaMemcpyDeviceToHost, st));
+  G_CUDA(cudaStreamSynchronize(st));
+  return SGTD_OK;
+}
+
+// One wave of a sharded call: this rank aligns the problems whose target it holds (tgt set: its own keyframes),
+// then one all-reduce hands every rank every problem's ProbOut and an "aligned" word (1: its owner aligned it).
+static_assert(sizeof(ProbOut) % 4 == 0, "ProbOut packs into 32-bit words");
+constexpr size_t kOutWords = sizeof(ProbOut) / 4 + 1;
+static int solve_wave_sharded(sgtd_handle *h, GicpPool &P, const std::vector<ProbIn> &in, int k, const sgtd_gicp_params &prm,
+                              std::vector<ProbOut> &out) {
+  std::vector<ProbIn> mine;
+  std::vector<size_t> at;
+  for (size_t i = 0; i < in.size(); ++i)
+    if (in[i].tgt) { mine.push_back(in[i]); at.push_back(i); }
+  std::vector<ProbOut> res;
+  if (int rc = solve_problems(h, P, mine, k, prm, res)) return rc;
+  std::vector<uint32_t> w(in.size() * kOutWords, 0u);
+  for (size_t j = 0; j < at.size(); ++j) {
+    std::memcpy(&w[at[j] * kOutWords], &res[j], sizeof(ProbOut));
+    w[at[j] * kOutWords + kOutWords - 1] = 1u;
+  }
+  if (int rc = allreduce_words(h, P, w)) return rc;
+  out.assign(in.size(), ProbOut{});
+  for (size_t i = 0; i < in.size(); ++i) {
+    // every rank sees the same sums, so a problem with no owner (or two) fails on every rank alike
+    if (w[i * kOutWords + kOutWords - 1] != 1u)
+      return sgtd_fail(h, SGTD_E_INVALID, "gicp_refine_batch: ranks disagree on a candidate's owner (same arguments and options on every rank?)", __FILE__, __LINE__);
+    std::memcpy(&out[i], &w[i * kOutWords], sizeof(ProbOut));
   }
   return SGTD_OK;
 }
@@ -1048,6 +1096,7 @@ extern "C" int sgtd_gicp_refine_batch(sgtd_handle *h, const float *sources_xyz, 
   const int k = prm->num_neighbors;
   DeviceScope ds(h->device);
   GicpPool &P = pool_of(h);
+  // arguments that are the same on every rank
   std::vector<QueryIn> Q(nq);
   int64_t total = 0;
   for (int32_t q = 0; q < nq; ++q) {
@@ -1057,24 +1106,50 @@ extern "C" int sgtd_gicp_refine_batch(sgtd_handle *h, const float *sources_xyz, 
       const int32_t c = order ? order[(int64_t)q * cand_stride + i] : i;
       if (c < 0 || c >= ncand[q]) return sgtd_fail(h, SGTD_E_INVALID, "gicp_refine_batch: order entry out of range", __FILE__, __LINE__);
       const sgtd_candidate &cd = cands[(int64_t)q * cand_stride + c];
-      if (cd.frame < 0) continue;
-      const auto it = P.frames.find((uint32_t)cd.frame);
-      if (it == P.frames.end()) continue;
-      if (k != P.store_k) return sgtd_fail(h, SGTD_E_INVALID, "gicp_refine_batch: num_neighbors differs from the stored clouds'", __FILE__, __LINE__);
-      if (ns < k || ns > 65535LL * kGicpThreads)
-        return sgtd_fail(h, SGTD_E_INVALID, "gicp_refine_batch: a source has fewer points than num_neighbors", __FILE__, __LINE__);
-      Q[q].visit.push_back({c, it->second, &cd});
+      if (cd.frame >= 0) Q[q].visit.push_back({c, nullptr, &cd});
     }
     Q[q].ns = (int32_t)ns;
     total = std::max(total, src_offsets[q + 1]);
   }
-  const float *d_src = nullptr;
-  if (total > 0) {
-    if (!sources_xyz) return sgtd_fail(h, SGTD_E_INVALID, "null argument", __FILE__, __LINE__);
-    if (int rc = device_source(h, P, sources_xyz, total, P.in_xyz, &d_src)) return rc;
+  if (total > 0 && !sources_xyz) return sgtd_fail(h, SGTD_E_INVALID, "null argument", __FILE__, __LINE__);
+  // Presence of every candidate's cloud, one word per candidate slot.  On a handle with a communicator only the
+  // rank owning cand.frame looks it up, and one sum all-reduce tells every rank what the owners hold (and whether
+  // the call fails) before any alignment.
+  const bool sharded = h->nranks > 1 && h->nccl;
+  constexpr uint32_t kHeld = 1, kBadK = 2, kBadSource = 4;
+  std::vector<uint32_t> pres((size_t)nq * cand_stride, 0u);
+  bool mine = false;
+  for (int32_t q = 0; q < nq; ++q) {
+    const int64_t ns = src_offsets[q + 1] - src_offsets[q];
+    for (Visit &v : Q[q].visit) {
+      if (sharded && !h->owns_frame(v.cd->frame)) continue;
+      const auto it = P.frames.find((uint32_t)v.cd->frame);
+      if (it == P.frames.end()) continue;
+      v.tgt = it->second;
+      mine = true;
+      pres[(size_t)q * cand_stride + v.c] = kHeld | (k != P.store_k ? kBadK : 0u) | (ns < k || ns > 65535LL * kGicpThreads ? kBadSource : 0u);
+    }
   }
+  if (sharded)
+    if (int rc = allreduce_words(h, P, pres)) return rc;
+  for (int32_t q = 0; q < nq; ++q) {
+    std::vector<Visit> held;
+    for (const Visit &v : Q[q].visit) {
+      const uint32_t w = pres[(size_t)q * cand_stride + v.c];
+      if (w & kBadK) return sgtd_fail(h, SGTD_E_INVALID, "gicp_refine_batch: num_neighbors differs from the stored clouds'", __FILE__, __LINE__);
+      if (w & kBadSource) return sgtd_fail(h, SGTD_E_INVALID, "gicp_refine_batch: a source has fewer points than num_neighbors", __FILE__, __LINE__);
+      if (w & kHeld) held.push_back(v);  // tgt stays NULL where another rank holds the cloud
+    }
+    Q[q].visit.swap(held);
+  }
+  const float *d_src = nullptr;
+  if (mine)
+    if (int rc = device_source(h, P, sources_xyz, total, P.in_xyz, &d_src)) return rc;
   for (int32_t q = 0; q < nq; ++q) Q[q].xyz = d_src ? d_src + 3 * src_offsets[q] : nullptr;
-  return refine_queries(h, P, Q, k, *prm, chosen, transformation12, fitness, n_aligned);
+  SolveWave solve;
+  if (sharded)
+    solve = [&](const std::vector<ProbIn> &in, std::vector<ProbOut> &out) { return solve_wave_sharded(h, P, in, k, *prm, out); };
+  return refine_queries(h, P, Q, k, *prm, chosen, transformation12, fitness, n_aligned, nullptr, solve);
 }
 
 extern "C" int sgtd_gicp_refine_stats(const sgtd_handle *h, int64_t *problems, int32_t *waves, int32_t *rounds) {

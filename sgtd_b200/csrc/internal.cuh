@@ -206,7 +206,10 @@ struct sgtd_handle {
   void (*s1pool_free)(void *) = nullptr;
   void *gicp_pool = nullptr;              // GICP temporaries (gicp.cu)
   void (*gicp_pool_free)(void *) = nullptr;
+  // keyframe ids this rank owns: [frame_lo(), frame_hi()), the sgtd_shard_init ranges; the last rank's is open-ended
   int64_t frame_lo() const { return frames_per_rank ? (int64_t)rank * frames_per_rank : 0; }
+  int64_t frame_hi() const { return frames_per_rank && rank < nranks - 1 ? frame_lo() + frames_per_rank : (1ll << 40); }
+  bool owns_frame(int64_t f) const { return f >= frame_lo() && f < frame_hi(); }
   int64_t frames_local() const { return (int64_t)frame_off.size() - 1; }
 };
 
