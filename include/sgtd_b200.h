@@ -173,7 +173,8 @@ int64_t sgtd_kernel_launches(const sgtd_handle *h);   /* kernels launched so far
  * "collect_mode" (0 auto, 1 inverted, 2 per-descriptor), "collect_group", "debug_novote",
  * "join_impl" (1 default; 0 / 2 experimental joins on 8-byte entries), "join_parts" (2..4: keyframe-range
  * passes inside a query group), "join_hint" (vote REDs with an L2 evict-last policy), "collect_unroll",
- * "verify_impl", "stats_unique", "s1_trace", "s1_replay" (1 = sequential stage-1 replay forms only; default 0 =
+ * "verify_impl", "region_vote" (sgtd_search_near: 0 auto, 1 dense join + mask, 2 sparse per allowed
+ * keyframe where the batch fits it), "stats_unique", "s1_trace", "s1_replay" (1 = sequential stage-1 replay forms only; default 0 =
  * component-parallel replay), "s1_rows", "s1_table", "gicp_wave", "gicp_cell_um" (see sgtd_gicp_map_add);
  * "s1_variant" (1 = class tables of local_map_creation) is the one that selects behaviour.  The same
  * switches are read once from the environment by sgtd_create (SGTD_VOTE_MODE=stream, SGTD_JOIN_GROUPS,
@@ -217,6 +218,26 @@ uint64_t sgtd_db_key(const sgtd_config *cfg, const sgtd_desc *d);
  * frame == current_frame_id_ (the reference's convention). */
 int sgtd_search(sgtd_handle *h, const sgtd_desc_batch *queries,
                 sgtd_search_result **out);
+/* Map-frame positions of keyframes [0, n): 3 doubles each (e.g. the translations
+ * of the map_poses12 given to sgtd_recall_rank), host or device pointer.  A call
+ * replaces the previous one; keyframes >= n have no position.  Any non-finite
+ * value: SGTD_E_INVALID.  On a sharded handle every rank is given the same array
+ * and keeps its own range.  Positions are not part of sgtd_db_save. */
+int sgtd_frame_positions(sgtd_handle *h, const double *xyz, int64_t n);
+/* Region search: sgtd_search with query q restricted to the keyframes f that
+ * have a position p with (dx*dx + dy*dy) + dz*dz <= r*r (double, no contraction),
+ * d = p - prior_xyz[3q..3q+2], r = radius[q] (+INFINITY: every keyframe with a
+ * position).  The result is what SearchLoop returns against a database holding
+ * only those keyframes, with ids unchanged: votes, ranking, match and inlier
+ * lists, poses, loop result; the sgtd_result_* calls work on it as usual.  In
+ * sgtd_result_stats, M counts the votes cast on allowed keyframes; Q and P are
+ * the batch's; E and Pfound depend on the vote formulation (INTEGRATION.md).
+ * Collective on a handle with a communicator, like sgtd_search.  Host or device
+ * pointers; SGTD_E_INVALID for a NaN or negative radius, a non-finite prior, or
+ * no sgtd_frame_positions call before. */
+int sgtd_search_near(sgtd_handle *h, const sgtd_desc_batch *queries,
+                     const double *prior_xyz, const double *radius,
+                     sgtd_search_result **out);
 int32_t sgtd_result_queries(const sgtd_search_result *r);
 /* loops: nq entries; cands: nq * candidate_num entries (entry c of query q at
  * q*candidate_num + c, valid for c < loops[q].ncand).  Either may be NULL. */

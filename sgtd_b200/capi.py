@@ -82,6 +82,8 @@ SYMBOLS = {
     "sgtd_finalize_db": (C.c_int, [_VP]),
     "sgtd_db_key": (C.c_uint64, [C.POINTER(Config), _VP]),
     "sgtd_search": (C.c_int, [_VP, _VP, C.POINTER(_VP)]),
+    "sgtd_frame_positions": (C.c_int, [_VP, _VP, _I64]),
+    "sgtd_search_near": (C.c_int, [_VP, _VP, _VP, _VP, C.POINTER(_VP)]),
     "sgtd_result_queries": (_I32, [_VP]),
     "sgtd_result_download": (C.c_int, [_VP, _VP, _VP, _VP]),
     "sgtd_result_matches": (C.c_int, [_VP, _VP, _I32, _I32, _VP, _VP, _VP, _I64]),
@@ -462,6 +464,25 @@ class STDescManager:
     def search(self, batch):
         out = C.c_void_p()
         self._chk(lib().sgtd_search(self._h, batch.ptr, C.byref(out)))
+        return SearchResult(self, out)
+
+    def frame_positions(self, xyz):
+        """Map-frame positions of keyframes [0, n): float64 [n, 3] (host array or raw device pointer with n given
+        as xyz=(ptr, n)); a call replaces the previous one."""
+        if isinstance(xyz, tuple):
+            ptr, n = xyz
+        else:
+            xyz = np.ascontiguousarray(xyz, np.float64).reshape(-1, 3)
+            ptr, n = xyz, xyz.shape[0]
+        self._chk(lib().sgtd_frame_positions(self._h, _p(ptr), n))
+
+    def search_near(self, batch, prior_xyz, radius):
+        """search() with query q restricted to the keyframes within radius[q] of prior_xyz[q] (float64 [nq, 3],
+        [nq]; np.inf: every keyframe with a position)."""
+        prior = np.ascontiguousarray(prior_xyz, np.float64).reshape(-1, 3)
+        rad = np.ascontiguousarray(radius, np.float64).reshape(-1)
+        out = C.c_void_p()
+        self._chk(lib().sgtd_search_near(self._h, batch.ptr, _p(prior), _p(rad), C.byref(out)))
         return SearchResult(self, out)
 
     def db_fetch(self, g):

@@ -1,5 +1,6 @@
 // api.cu -- the extern "C" surface of libsgtd_b200.so (see include/sgtd_b200.h).
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -250,6 +251,7 @@ int sgtd_set_option(sgtd_handle *h, const char *name, int32_t value) {
   else if (!strcmp(name, "s1_table")) h->opt.s1_table = value == 1;
   else if (!strcmp(name, "gicp_wave")) h->opt.gicp_wave = std::max(0, (int)value);
   else if (!strcmp(name, "gicp_cell_um")) h->opt.gicp_cell_um = std::max(0, (int)value);
+  else if (!strcmp(name, "region_vote")) h->opt.region_vote = (value >= 0 && value <= 2) ? (int)value : 0;
   else SGTD_FAIL(h, SGTD_E_INVALID, "unknown option");
   return SGTD_OK;
 }
@@ -262,6 +264,7 @@ int sgtd_destroy(sgtd_handle *h) {
   h->rec.release(); h->vert.release(); h->d_frame_off.release();
   h->v_s0.release(); h->v_s1.release(); h->v_s2.release(); h->v_frame.release(); h->v_pack.release(); h->v_pack8.release();
   h->table.release(); h->v_cut.release(); h->f_key.release(); h->f_g.release(); h->f_side.release(); h->scratch.release(); h->stage_in.release(); h->uniq_bitmap.release();
+  h->pos.release(); h->region_q.release(); h->region_items.release();
   if (h->s1pool && h->s1pool_free) h->s1pool_free(h->s1pool);
   if (h->gicp_pool && h->gicp_pool_free) h->gicp_pool_free(h->gicp_pool);
   for (auto *r : h->result_pool) destroy_result(r);
@@ -471,6 +474,70 @@ int sgtd_search(sgtd_handle *h, const sgtd_desc_batch *queries, sgtd_search_resu
   h->live_results.insert(r);
   int rc = search(h, queries, r);
   if (rc) { sgtd_result_free(r); return rc; }
+  *out = r;
+  return SGTD_OK;
+}
+
+// host copy of n doubles the caller passed as a host or device pointer
+static int fetch_doubles(sgtd_handle *h, const double *src, size_t n, std::vector<double> &out) {
+  out.resize(n);
+  if (n == 0) return SGTD_OK;
+  if (is_device_ptr(src)) SGTD_CUDA(h, cudaMemcpy(out.data(), src, n * 8, cudaMemcpyDeviceToHost));
+  else memcpy(out.data(), src, n * 8);
+  return SGTD_OK;
+}
+
+int sgtd_frame_positions(sgtd_handle *h, const double *xyz, int64_t n) {
+  if (!h || n < 0 || (n > 0 && !xyz)) SGTD_FAIL(h, SGTD_E_INVALID, "bad argument");
+  SetDevice sd(h->device);
+  std::vector<double> p;
+  int rc = fetch_doubles(h, xyz, (size_t)n * 3, p);
+  if (rc) return rc;
+  for (double v : p)
+    if (!std::isfinite(v)) SGTD_FAIL(h, SGTD_E_INVALID, "non-finite keyframe position");
+  // this rank keeps the positions of its own keyframe range
+  const int64_t lo = h->frame_lo(), hi = std::min<int64_t>(n, h->frame_hi());
+  const int64_t nloc = std::max<int64_t>(0, hi - lo);
+  if (nloc > 0) {
+    SGTD_CUDA(h, h->pos.reserve((size_t)nloc * 3, h->stream, false));
+    SGTD_CUDA(h, cudaMemcpyAsync(h->pos.p, p.data() + 3 * lo, (size_t)nloc * 24, cudaMemcpyHostToDevice, h->stream));
+    SGTD_CUDA(h, cudaStreamSynchronize(h->stream));
+  }
+  h->n_pos = nloc;
+  h->pos_set = true;
+  return SGTD_OK;
+}
+
+int sgtd_search_near(sgtd_handle *h, const sgtd_desc_batch *queries, const double *prior_xyz, const double *radius,
+                     sgtd_search_result **out) {
+  if (!h || !queries || !out) SGTD_FAIL(h, SGTD_E_INVALID, "bad argument");
+  *out = nullptr;
+  const int nq = queries->nscans;
+  if (nq > 0 && (!prior_xyz || !radius)) SGTD_FAIL(h, SGTD_E_INVALID, "bad argument");
+  if (!h->pos_set) SGTD_FAIL(h, SGTD_E_INVALID, "no keyframe positions set (sgtd_frame_positions)");
+  SetDevice sd(h->device);
+  std::vector<double> c, rad;
+  int rc = fetch_doubles(h, prior_xyz, (size_t)nq * 3, c);
+  if (!rc) rc = fetch_doubles(h, radius, (size_t)nq, rad);
+  if (rc) return rc;
+  std::vector<double> reg((size_t)std::max(nq, 1) * 4);
+  for (int q = 0; q < nq; ++q) {
+    if (!(rad[q] >= 0.0)) SGTD_FAIL(h, SGTD_E_INVALID, "radius must be >= 0 (NaN is not)");
+    for (int i = 0; i < 3; ++i) {
+      if (!std::isfinite(c[3 * q + i])) SGTD_FAIL(h, SGTD_E_INVALID, "non-finite position prior");
+      reg[4 * q + i] = c[3 * q + i];
+    }
+    reg[4 * q + 3] = rad[q];
+  }
+  SGTD_CUDA(h, h->region_q.reserve(reg.size(), h->stream, false));
+  SGTD_CUDA(h, cudaMemcpyAsync(h->region_q.p, reg.data(), reg.size() * 8, cudaMemcpyHostToDevice, h->stream));
+  sgtd_search_result *r;
+  if (!h->result_pool.empty()) { r = h->result_pool.back(); h->result_pool.pop_back(); }
+  else r = new sgtd_search_result();
+  r->h = h;
+  h->live_results.insert(r);
+  rc = search(h, queries, r, true);
+  if (rc) { cudaStreamSynchronize(h->stream); sgtd_result_free(r); return rc; }
   *out = r;
   return SGTD_OK;
 }

@@ -157,6 +157,7 @@ struct sgtd_options {
                           // (bulk-async staged tiles).  Measured on the bench workload: 9.0 / 11.4 / 12.6 ms.
   int gicp_wave = 0;      // candidates per query and GICP wave (0: automatic, 1, 2, 4, ... per wave)
   int gicp_cell_um = 0;   // cell size of the nearest-neighbour grids built from now on, micrometres (0: automatic)
+  int region_vote = 0;    // sgtd_search_near's vote formulation: 0 automatic, 1 dense (join + mask), 2 sparse (where it fits)
 };
 
 struct sgtd_handle {
@@ -193,6 +194,12 @@ struct sgtd_handle {
   sgtd::DevBuf<uint64_t> f_key;
   sgtd::DevBuf<uint32_t> f_g;
   sgtd::DevBuf<double> f_side;  // side lengths in frame-view order, 3 per entry
+  // keyframe positions (sgtd_frame_positions): local keyframes [0, n_pos) of this rank, 3 doubles each
+  sgtd::DevBuf<double> pos;
+  int64_t n_pos = 0;
+  bool pos_set = false;
+  sgtd::DevBuf<double> region_q;        // sgtd_search_near: {cx, cy, cz, r} per query of the running call
+  sgtd::DevBuf<uint32_t> region_items;  // sgtd_search_near: allowed keyframes of every query (sparse vote)
   // scratch + recycled objects: steady-state build/search calls do no cudaMalloc/cudaFree
   sgtd::DevBuf<uint32_t> uniq_bitmap;
   sgtd::DevBuf<unsigned char> scratch;
@@ -229,7 +236,8 @@ namespace sgtd {
 int build_descriptors(sgtd_handle *h, const sgtd_node *d_nodes, const std::vector<int64_t> &off,
                       const std::vector<uint32_t> &frame_ids, sgtd_desc_batch *out);
 int finalize_db(sgtd_handle *h);
-int search(sgtd_handle *h, const sgtd_desc_batch *q, sgtd_search_result *r);
+// region = true: sgtd_search_near, the queries' regions in h->region_q
+int search(sgtd_handle *h, const sgtd_desc_batch *q, sgtd_search_result *r, bool region = false);
 void merge_topk_host(const int32_t *votes, const int32_t *frames, int nlists, int k,
                      int32_t *out_votes, int32_t *out_frames);
 }  // namespace sgtd

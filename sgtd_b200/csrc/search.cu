@@ -1324,11 +1324,15 @@ constexpr int kIndexThreads = 1024;
 // inserts every probe with one CAS.
 __global__ void __launch_bounds__(kIndexThreads) k_query_index(const DescRec *q, const QAux *aux, const int64_t *q_off,
                                                                int q_base, uint32_t *qt, uint32_t stride,
-                                                               const uint32_t *qprobes, const sgtd_candidate *cands, int k) {
+                                                               const uint32_t *qprobes, const sgtd_candidate *cands, int k,
+                                                               const int64_t *region_off) {
   const int qi = q_base + blockIdx.x;  // tables are indexed by the query's position inside its group
-  // a query none of whose candidates is materialised on this rank (sharded database: the candidates of a
-  // query cluster in one or two keyframe-range shards) needs no table
-  {
+  if (region_off) {
+    // region vote (k_region_vote): the query needs its table when it has allowed keyframes on this rank
+    if (region_off[qi + 1] == region_off[qi]) return;
+  } else {
+    // a query none of whose candidates is materialised on this rank (sharded database: the candidates of a
+    // query cluster in one or two keyframe-range shards) needs no table
     __shared__ int s_any;
     if (threadIdx.x == 0) s_any = 0;
     __syncthreads();
@@ -1559,6 +1563,129 @@ __global__ void __launch_bounds__(kCollectThreads, kMinBlocks) k_collect_inv(Col
     P.m_cell[c.match_off + i] = (uint8_t)((rec >> 12) & 31u);
     P.m_g[c.match_off + i] = P.f_g[fo + (int64_t)(rec & 0xFFFu)];
   }
+}
+
+// ============================ region search (sgtd_search_near) =======================
+// A query q may only vote for the keyframes f of its region: f has a position p (sgtd_frame_positions) and
+// (dx*dx + dy*dy) + dz*dz <= r*r with d = p - c_q, in double without contraction.  Votes depend on each
+// keyframe's own descriptors only, and a bucket restricted to some keyframes keeps its insertion order, so
+// the vote rows with every other entry at zero are the rows of a database holding only those keyframes;
+// top-k, collect and verification downstream run unchanged on them.
+constexpr int kRegionThreads = 256;
+
+// qreg: {cx, cy, cz, r} per query
+__device__ __forceinline__ bool region_allowed(const double *pos, int64_t npos, int64_t f, const double *qreg) {
+  if (f >= npos) return false;  // no stored position
+  const double dx = __dsub_rn(pos[3 * f], qreg[0]), dy = __dsub_rn(pos[3 * f + 1], qreg[1]), dz = __dsub_rn(pos[3 * f + 2], qreg[2]);
+  return __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)) <= __dmul_rn(qreg[3], qreg[3]);
+}
+
+// One CTA per query: allowed keyframes of this rank (cnt[q]) and the vote-index entries they hold (summed
+// into *entries, what the host weighs the two vote formulations by).
+__global__ void __launch_bounds__(kRegionThreads) k_region_count(const double *pos, int64_t npos, int64_t F, const double *qreg,
+                                                                 const int64_t *frame_off, int64_t *cnt,
+                                                                 unsigned long long *entries) {
+  __shared__ unsigned long long s_sum[2][kRegionThreads / 32];
+  const int q = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  unsigned long long n = 0, e = 0;
+  for (int64_t f = threadIdx.x; f < F; f += kRegionThreads)
+    if (region_allowed(pos, npos, f, qreg + 4 * q)) { ++n; e += (unsigned long long)(frame_off[f + 1] - frame_off[f]); }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) { n += __shfl_xor_sync(0xffffffffu, n, o); e += __shfl_xor_sync(0xffffffffu, e, o); }
+  if (lane == 0) { s_sum[0][wid] = n; s_sum[1][wid] = e; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long tn = 0, te = 0;
+    for (int w = 0; w < kRegionThreads / 32; ++w) { tn += s_sum[0][w]; te += s_sum[1][w]; }
+    cnt[q] = (int64_t)tn;
+    if (te) atomicAdd(entries, te);
+  }
+}
+
+// One CTA per query: its allowed keyframes in ascending order at items[off[q] ..) (ordered compaction), and
+// the Q / P statistics of the query (the sparse formulation has no probe emission to count them).
+__global__ void __launch_bounds__(kRegionThreads) k_region_fill(const double *pos, int64_t npos, int64_t F, const double *qreg,
+                                                                const int64_t *off, uint32_t *items, const int64_t *q_off,
+                                                                const uint32_t *qprobes, unsigned long long *counters) {
+  __shared__ uint32_t s_warp[kRegionThreads / 32];
+  const int q = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  int64_t base = off[q];
+  for (int64_t f0 = 0; f0 < F; f0 += kRegionThreads) {
+    const int64_t f = f0 + threadIdx.x;
+    const bool ok = f < F && region_allowed(pos, npos, f, qreg + 4 * q);
+    const unsigned bal = __ballot_sync(0xffffffffu, ok);
+    if (lane == 0) s_warp[wid] = __popc(bal);
+    __syncthreads();
+    uint32_t before = 0, total = 0;
+#pragma unroll
+    for (int w = 0; w < kRegionThreads / 32; ++w) { before += w < wid ? s_warp[w] : 0u; total += s_warp[w]; }
+    if (ok) items[base + before + __popc(bal & ((1u << lane) - 1u))] = (uint32_t)f;
+    base += total;
+    __syncthreads();  // s_warp is rewritten by the next chunk
+  }
+  if (threadIdx.x == 0) {
+    atomicAdd(counters + 0, (unsigned long long)(q_off[q + 1] - q_off[q]));
+    atomicAdd(counters + 1, (unsigned long long)qprobes[q]);
+  }
+}
+
+// Dense formulation: the unrestricted vote rows, then every entry of a keyframe outside the query's region
+// set to zero (before k_topk, so that its match count covers the allowed keyframes only).
+__global__ void __launch_bounds__(kRegionThreads) k_region_mask(const double *pos, int64_t npos, int64_t F, const double *qreg,
+                                                                uint32_t *votes) {
+  const int q = blockIdx.x;
+  uint32_t *row = votes + (size_t)q * (size_t)F;
+  for (int64_t f = (int64_t)blockIdx.y * kRegionThreads + threadIdx.x; f < F; f += (int64_t)gridDim.y * kRegionThreads)
+    if (!region_allowed(pos, npos, f, qreg + 4 * q)) row[f] = 0u;
+}
+
+// Sparse formulation: one warp per (query, allowed keyframe).  The warp looks every entry of the keyframe's
+// key-sorted view up in the query's probe multimap (k_query_index) and counts the matches with
+// k_collect_inv's tests -- exact key, keyframe other than the query's, FP64 rough distance -- i.e. exactly
+// the votes the probe-major kernels cast for that keyframe: each (descriptor, probe, entry) triple with
+// equal keys is one slot-entry pair of the multimap.  It only counts, so no list capacity applies.
+__global__ void __launch_bounds__(kRegionThreads) k_region_vote(const uint32_t *items, const int64_t *off, int nq, int64_t i0,
+                                                                int64_t i1, int q_base, const DescRec *q, const QAux *aux,
+                                                                const int64_t *q_off, const uint32_t *qt, uint32_t stride,
+                                                                const uint32_t *qprobes, const int64_t *frame_off,
+                                                                const uint64_t *f_key, const double *f_side, uint32_t frame_lo,
+                                                                int64_t F, uint32_t *votes, unsigned long long *counters) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = ((int64_t)blockIdx.x * kRegionThreads + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * kRegionThreads) >> 5;
+  unsigned long long cE = 0;
+  for (int64_t it = i0 + warp; it < i1; it += nwarps) {
+    int lo = 0, hi = nq - 1;  // the query of the item: last q with off[q] <= it
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (off[mid] <= it) lo = mid; else hi = mid - 1; }
+    const int qi = lo;
+    const uint32_t f = items[it];
+    const int64_t fo = frame_off[f];
+    const int nf = (int)(frame_off[f + 1] - fo);
+    const int64_t q0 = q_off[qi];
+    const uint32_t *tk = qt + (size_t)(qi - q_base) * stride;
+    const uint32_t mask = qt_size(qprobes[qi], stride) - 1;
+    const uint32_t cframe = frame_lo + f;
+    uint32_t cnt = 0;
+    for (int p = lane; p < nf; p += 32) {
+      const uint64_t key = f_key[fo + p];
+      const unsigned long long hsh = mix64(key);
+      const uint32_t tag = qt_tag(hsh);
+      uint32_t ps = (uint32_t)hsh & mask;
+      for (uint32_t sl = __ldg(tk + ps); sl != kQtEmpty; ps = (ps + 1) & mask, sl = __ldg(tk + ps)) {
+        if ((sl >> 18) != tag) continue;
+        const uint32_t io = sl & 0x3FFFFu, i = io >> 5;
+        const DescRec r = q[q0 + i];
+        if (probe_cell_key(r, (int)(io & 31u)) != key || r.frame == cframe) continue;
+        const double *e = f_side + 3 * (fo + (int64_t)p);
+        const double d2 = sqn3(__dsub_rn(r.s[0], e[0]), __dsub_rn(r.s[1], e[1]), __dsub_rn(r.s[2], e[2]));
+        cnt += d2 < aux[q0 + i].thr2;
+      }
+    }
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if (lane == 0) votes[(size_t)qi * (size_t)F + f] = cnt;
+    cE += (unsigned long long)nf;
+  }
+  if (lane == 0 && cE) atomicAdd(counters + 3, cE);
 }
 
 // ============================ verification ===========================================
@@ -1979,7 +2106,11 @@ __global__ void k_best(const sgtd_candidate *cands, int nq, int k, double icp, s
 // ============================ host driver ================================================
 static float ev_ms(cudaEvent_t a, cudaEvent_t b) { float ms = 0; cudaEventElapsedTime(&ms, a, b); return ms; }
 
-int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r) {
+// Region search, automatic formulation: the sparse vote runs when the vote-index entries of the allowed
+// keyframes, summed over the batch, are below this share of (queries x entries on this rank).
+constexpr double kRegionSparseShare = 0.0015;
+
+int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, bool region) {
   cudaStream_t st = h->stream;
   int rc = finalize_db(h);
   if (rc) return rc;
@@ -2050,6 +2181,14 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r) {
   size_t o_jd = o; o += run_join ? al((size_t)std::max<int64_t>(qb->n, 1) * sizeof(JoinDesc)) : 0;
   size_t o_pose = o; o += al((size_t)std::max(nq * k, 1) * kMaxHyp * 12 * sizeof(double));
   size_t o_jcub = o; o += al(cubj);
+  // region search: per-query counts and offsets of the allowed keyframes, their entries, scan temp
+  const bool region_votes = region && nq > 0 && F > 0;
+  size_t cubr = 0;
+  if (region_votes) cub::DeviceScan::ExclusiveSum(nullptr, cubr, (int64_t *)nullptr, (int64_t *)nullptr, nq + 1, st);
+  size_t o_rcnt = o; o += region_votes ? al((size_t)(nq + 1) * 8) : 0;
+  size_t o_roff = o; o += region_votes ? al((size_t)(nq + 1) * 8) : 0;
+  size_t o_rent = o; o += region_votes ? al(8) : 0;
+  size_t o_rcub = o; o += region_votes ? al(cubr) : 0;
   SGTD_CUDA(h, h->scratch.reserve(o, st, false));
   unsigned char *S = h->scratch.p;
   int32_t *lv = (int32_t *)(S + o_lv), *lf = (int32_t *)(S + o_lf), *gv = (int32_t *)(S + o_gv);
@@ -2076,7 +2215,54 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r) {
   SGTD_CUDA(h, cudaMemsetAsync(r->votes.p, 0, (size_t)nq * Fa * 4, st));
   SGTD_CUDA(h, cudaMemsetAsync(r->counters.p, 0, 8 * 8, st));
   SGTD_CUDA(h, cudaEventRecord(ev[7], st));
-  if (nq > 0 && qb->n > 0 && h->rec.n > 0) {
+  // region search: allowed sets of this rank's keyframes, then the vote formulation.  The sparse one needs
+  // every query in the probe-multimap format (kInvMaxDesc descriptors at most).
+  bool sparse = false, tables_ready = false;
+  std::vector<int64_t> roff;
+  const int64_t npos = std::min<int64_t>(h->n_pos, F);
+  int64_t *d_roff = (int64_t *)(S + o_roff);
+  if (region_votes) {
+    int64_t *d_rcnt = (int64_t *)(S + o_rcnt);
+    unsigned long long *d_rent = (unsigned long long *)(S + o_rent), ent = 0;
+    SGTD_CUDA(h, cudaMemsetAsync(d_rent, 0, 8, st));
+    SGTD_CUDA(h, cudaMemsetAsync(d_rcnt + nq, 0, 8, st));
+    k_region_count<<<nq, kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, h->d_frame_off.p, d_rcnt, d_rent);
+    SGTD_LAUNCHED(h);
+    SGTD_CUDA(h, cub::DeviceScan::ExclusiveSum(S + o_rcub, cubr, d_rcnt, d_roff, nq + 1, st));
+    SGTD_LAUNCHED(h);
+    roff.resize((size_t)nq + 1);
+    SGTD_CUDA(h, cudaMemcpyAsync(roff.data(), d_roff, (size_t)(nq + 1) * 8, cudaMemcpyDeviceToHost, st));
+    SGTD_CUDA(h, cudaMemcpyAsync(&ent, d_rent, 8, cudaMemcpyDeviceToHost, st));
+    SGTD_CUDA(h, cudaStreamSynchronize(st));
+    const bool fits = qb->n > 0 && h->rec.n > 0 && max_dq <= kInvMaxDesc;
+    const bool small = (double)ent < kRegionSparseShare * (double)nq * (double)h->rec.n;
+    sparse = fits && (h->opt.region_vote == 2 || (h->opt.region_vote == 0 && small));
+  }
+  if (sparse) {
+    const int64_t nitems = roff[nq];
+    SGTD_CUDA(h, h->region_items.reserve((size_t)std::max<int64_t>(nitems, 1), st, false));
+    k_region_fill<<<nq, kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, d_roff, h->region_items.p, qb->d_off.p,
+                                                 (const uint32_t *)(S + o_qpr), r->counters.p);
+    SGTD_LAUNCHED(h);
+    for (int qb0 = 0; qb0 < nq; qb0 += qt_group) {
+      const int gq = std::min(qt_group, nq - qb0);
+      const int64_t i0 = roff[qb0], i1 = roff[qb0 + gq];
+      if (i1 == i0) continue;
+      k_query_index<<<gq, kIndexThreads, 0, st>>>(qb->rec.p, aux, qb->d_off.p, qb0, (uint32_t *)(S + o_qtk), qt_ts,
+                                                  (const uint32_t *)(S + o_qpr), r->cands.p, k, d_roff);
+      SGTD_LAUNCHED(h);
+      const int rgrid = (int)std::min<int64_t>((i1 - i0 + kRegionThreads / 32 - 1) / (kRegionThreads / 32), (int64_t)h->sm_count * 8);
+      k_region_vote<<<rgrid, kRegionThreads, 0, st>>>(h->region_items.p, d_roff, nq, i0, i1, qb0, qb->rec.p, aux, qb->d_off.p,
+                                                      (const uint32_t *)(S + o_qtk), qt_ts, (const uint32_t *)(S + o_qpr),
+                                                      h->d_frame_off.p, h->f_key.p, h->f_side.p, (uint32_t)h->frame_lo(), Fa,
+                                                      r->votes.p, r->counters.p);
+      SGTD_LAUNCHED(h);
+      SGTD_CUDA(h, cudaGetLastError());
+    }
+    tables_ready = qt_group >= nq;  // the collect below finds every table it needs already built
+    m_by_topk = true;
+  }
+  if (nq > 0 && qb->n > 0 && h->rec.n > 0 && !sparse) {
     VoteParams V{};
     V.perm = sort_q ? (const uint32_t *)(S + o_si1) : nullptr;
     V.q = qb->rec.p; V.aux = aux; V.q_off = qb->d_off.p; V.nq = nq; V.nd = qb->n;
@@ -2193,6 +2379,16 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r) {
         join_timed = true;
       }
     }
+    if (region_votes) {
+      // dense formulation of a region search: clear the votes outside each query's region; the matches
+      // are then counted by k_topk over the allowed keyframes (whatever the vote kernel counted is dropped)
+      k_region_mask<<<dim3((unsigned)nq, (unsigned)std::min<int64_t>((F + kRegionThreads - 1) / kRegionThreads, 65535)),
+                      kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, r->votes.p);
+      SGTD_LAUNCHED(h);
+      SGTD_CUDA(h, cudaGetLastError());
+      SGTD_CUDA(h, cudaMemsetAsync(r->counters.p + 4, 0, 8, st));
+      m_by_topk = true;
+    }
   }
   SGTD_CUDA(h, cudaEventRecord(ev[1], st));
   const int vote_launches = (int)(h->launches - launches0);
@@ -2254,15 +2450,18 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r) {
       SGTD_CUDA(h, cudaFuncSetAttribute(k_collect_inv<1, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, inv_smem_max));
       for (int qb0 = 0; qb0 < nq; qb0 += qt_group) {
         const int gq = std::min(qt_group, nq - qb0);
-        k_query_index<<<gq, kIndexThreads, 0, st>>>(qb->rec.p, aux, qb->d_off.p, qb0, (uint32_t *)(S + o_qtk), qt_ts,
-                                                    (const uint32_t *)(S + o_qpr), r->cands.p, k);
+        if (!tables_ready) {
+          k_query_index<<<gq, kIndexThreads, 0, st>>>(qb->rec.p, aux, qb->d_off.p, qb0, (uint32_t *)(S + o_qtk), qt_ts,
+                                                      (const uint32_t *)(S + o_qpr), r->cands.p, k, nullptr);
+          SGTD_LAUNCHED(h);
+        }
         I.q_base = qb0;
         // (measured on the bench workload: 1 hit per thread and trip at 4 CTAs/SM 5.0 ms, 2 hits at 3 CTAs/SM 5.6,
         // 4 hits at 2 CTAs/SM 7.2; 1 hit at 5 / 6 CTAs/SM (48 / 40 registers) 5.0 / 5.5 -- occupancy wins up to 4)
         if (h->opt.collect_unroll == 4) k_collect_inv<4, 2><<<(unsigned)gq * k, kCollectThreads, inv_smem, st>>>(I);
         else if (h->opt.collect_unroll == 2) k_collect_inv<2, 3><<<(unsigned)gq * k, kCollectThreads, inv_smem, st>>>(I);
         else k_collect_inv<1, 4><<<(unsigned)gq * k, kCollectThreads, inv_smem, st>>>(I);
-        h->launches += 2;
+        SGTD_LAUNCHED(h);
       }
     }
     CollectParams C{};
