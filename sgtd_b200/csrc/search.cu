@@ -15,6 +15,7 @@
 // outcome: "sqrt(x) < t" is evaluated as "x < sq_threshold(t)".
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cuda/atomic>
 #include <cstdlib>
 #include <cstring>
 
@@ -1689,7 +1690,7 @@ __global__ void __launch_bounds__(kRegionThreads) k_region_vote(const uint32_t *
 }
 
 // ============================ verification ===========================================
-constexpr int kVerifyThreads = 128;
+constexpr int kVerifyThreads = 128, kVerifyCtas = 5;  // k_verify: 4 warps per CTA, 5 CTAs per SM (shared memory)
 
 __device__ __forceinline__ double dot3s(double a0, double b0, double a1, double b1, double a2, double b2) {
   return __dadd_rn(__dmul_rn(a0, b0), __dadd_rn(__dmul_rn(a1, b1), __dmul_rn(a2, b2)));  // e0 + (e1 + e2), see norm3
@@ -1818,17 +1819,79 @@ __device__ __forceinline__ uint32_t pair_hash(const uint32_t *w) {
 
 constexpr int kVotePlanes = 5;  // bit-sliced vote counters: a lane adds up to 2^5 - 1 match masks before a flush
 
-// adds a warp's bit-sliced counters (bit h of plane k: 2^k votes of hypothesis h) to the votes
+// transposes the 32 x 32 bit matrix whose row l is lane l's x: returns the word whose bit l is bit `lane` of lane l's x
+__device__ __forceinline__ uint32_t transpose32(uint32_t x, int lane) {
+  const uint32_t m[5] = {0x0000FFFFu, 0x00FF00FFu, 0x0F0F0F0Fu, 0x33333333u, 0x55555555u};
+#pragma unroll
+  for (int s = 0; s < 5; ++s) {
+    const int j = 16 >> s;
+    const uint32_t y = __shfl_xor_sync(0xffffffffu, x, j);
+    x = (lane & j) ? (x & ~m[s]) | ((y & ~m[s]) >> j) : (x & m[s]) | ((y & m[s]) << j);
+  }
+  return x;
+}
+
+// adds a warp's bit-sliced counters (bit h of plane k: 2^k votes of hypothesis h) to the votes.  Each plane is
+// transposed across the warp, so that lane h counts hypothesis h (and h + 32) with one popc per plane.
 __device__ __forceinline__ void flush_votes(unsigned long long *cnt, int H, int lane, int *s_vote) {
-  for (int h = 0; h < H; ++h) {
+  for (int half = 0; half < 2 && 32 * half < H; ++half) {
     int n = 0;
 #pragma unroll
-    for (int k = 0; k < kVotePlanes; ++k) n += (int)((cnt[k] >> h) & 1ull) << k;
-    n = __reduce_add_sync(0xffffffffu, n);
-    if (lane == 0 && n) atomicAdd(&s_vote[h], n);
+    for (int k = 0; k < kVotePlanes; ++k) n += __popc(transpose32((uint32_t)(cnt[k] >> (32 * half)), lane)) << k;
+    const int h = 32 * half + lane;
+    if (h < H && n) atomicAdd(&s_vote[h], n);
   }
 #pragma unroll
   for (int k = 0; k < kVotePlanes; ++k) cnt[k] = 0ull;
+}
+
+// The id of `key` (hash h) in k_verify's pair table, inserted if new; -1 when it is new and no id is left.
+// A position holds 0 (empty) or a word: bits 10-30 of the hash with bit 31 set, and the pair id in bits 0-9.
+// An insert reserves an id, writes its key and then publishes the word with a CAS on an empty position; the
+// release fence between the two and the acquire load of a word make a published id's key visible to whoever
+// reads the word.  A lost CAS leaves the id reserved and probes on with it; if the pair turns out to have been
+// published by another thread the id stays unused (a hole: it has a key, so phase 2 tests it, but no match
+// refers to it).  No thread waits for another: each step returns, or moves to the next position, or re-reads
+// a position that has just become non-empty, and at most `limit` < cap positions are ever filled.
+__device__ __forceinline__ int insert_pair(uint32_t *s_tab, uint32_t (*s_key)[6], int *s_npair, const uint32_t *key,
+                                           uint32_t h, int cap, int limit) {
+  const uint32_t tag = (h | 0x80000000u) & ~1023u;
+  int p = h & (cap - 1), u = -1;
+  for (;;) {
+    const uint32_t w = cuda::atomic_ref<uint32_t, cuda::thread_scope_block>(s_tab[p]).load(cuda::memory_order_acquire);
+    if (w == 0u) {
+      if (u < 0) {
+        u = atomicAdd(s_npair, 1);
+        if (u >= limit) return -1;
+#pragma unroll
+        for (int i = 0; i < 6; ++i) s_key[u][i] = key[i];
+        cuda::atomic_thread_fence(cuda::memory_order_release, cuda::thread_scope_block);
+      }
+      if (atomicCAS(&s_tab[p], 0u, tag | (uint32_t)u) == 0u) return u;
+      continue;  // another insert took the position: read its word
+    }
+    if ((w & ~1023u) == tag) {
+      const int id = (int)(w & 1023u);
+      bool eq = true;
+#pragma unroll
+      for (int i = 0; i < 6; ++i) eq = eq && s_key[id][i] == key[i];
+      if (eq) return id;
+    }
+    p = (p + 1) & (cap - 1);
+  }
+}
+
+// The id of `key` if the word at its home position (no probing) holds it, else -1; read as in insert_pair
+__device__ __forceinline__ int find_home(uint32_t *s_tab, const uint32_t (*s_key)[6], const uint32_t *key,
+                                         uint32_t h, int cap) {
+  const uint32_t w =
+      cuda::atomic_ref<uint32_t, cuda::thread_scope_block>(s_tab[h & (cap - 1)]).load(cuda::memory_order_acquire);
+  if (w == 0u || (w & ~1023u) != ((h | 0x80000000u) & ~1023u)) return -1;
+  const int id = (int)(w & 1023u);
+  bool eq = true;
+#pragma unroll
+  for (int i = 0; i < 6; ++i) eq = eq && s_key[id][i] == key[i];
+  return eq ? id : -1;
 }
 
 // One CTA (4 warps) per candidate.  The vertex test of candidate_verify depends on one query vertex, one DB
@@ -1837,23 +1900,28 @@ __device__ __forceinline__ void flush_votes(unsigned long long *cnt, int H, int 
 // vertex) pairs.  So the kernel
 //   1. maps each vertex slot of each match to a pair id: an open-addressing table in shared memory keyed on
 //      the bits of the six coordinates (equal bits give equal outcomes; the descriptors' label fields play
-//      no part), rounds of up to 128 matches, one per thread;
+//      no part).  Each warp maps its own matches, 32 at a time, without barriers: a pair found at its home
+//      position is taken directly (find_home); for the others, lanes holding the same pair agree first, so
+//      that one of them probes on or inserts it (insert_pair);
 //   2. tests every distinct pair against every hypothesis in FP64, in the reference's operation order
 //      (vertex_inlier), and keeps the outcomes as a 64-bit mask per pair;
 //   3. votes: a match is an inlier of h iff bit h of the AND of its three masks is set; each lane adds
 //      the masks of its matches into bit-sliced counters (a ripple-carry add of 64 one-bit counts at once).
 // The table holds kPairCap pairs and the per-match ids kChunkMatches matches; longer or more varied
-// candidates run in chunks (votes add up across chunks, the table starts over when it fills).  A candidate
-// that took one chunk reads its inlier list back from the masks, the others re-test the best hypothesis.
-__global__ void __launch_bounds__(kVerifyThreads, 4) k_verify(VerifyParams P) {
+// candidates run in chunks whose votes add up.  A match that finds no id left records its index with
+// atomicMin(s_stop), and its warp stops; a warp maps its matches in increasing order, so after the chunk's
+// barrier every match before s_stop has its ids.  Those are voted, and the next chunk maps the rest into a
+// cleared table (a chunk that mapped nothing is retried with its first match alone, which always fits).
+// A candidate that took one chunk reads its inlier list back from the masks, the others re-test the best
+// hypothesis.
+__global__ void __launch_bounds__(kVerifyThreads, kVerifyCtas) k_verify(VerifyParams P) {
   __shared__ __align__(16) double s_pose[kMaxHyp][12];  // exact (R,t) of every hypothesis
-  __shared__ uint32_t s_tag[kPairTab];                  // hash of the pair at a position, 0 = empty
-  __shared__ uint16_t s_uid[kPairTab];                  // pair id at a position
+  __shared__ uint32_t s_tab[kPairTab];                  // position -> 0 (empty) or hash tag | pair id
   __shared__ uint32_t s_key[kPairCap][6];               // pair id -> bits of (query vertex xyz, DB vertex xyz)
   __shared__ unsigned long long s_hm[kPairCap];         // pair id -> bit h: an inlier under hypothesis h
   __shared__ uint32_t s_ids[kChunkMatches];             // match of the chunk -> its three pair ids
   __shared__ int s_vote[kMaxHyp];
-  __shared__ int s_npair, s_best, s_cnt[64 * (kVerifyThreads / 32) + 1];
+  __shared__ int s_npair, s_stop, s_best, s_cnt[64 * (kVerifyThreads / 32) + 1];
   sgtd_candidate *cd = P.cands + blockIdx.x;
   const int64_t moff = cd->match_off;
   const int M = cd->nmatch;
@@ -1864,88 +1932,77 @@ __global__ void __launch_bounds__(kVerifyThreads, 4) k_verify(VerifyParams P) {
   const int skip = M / 50 + 1;
   const int H = M / skip;
   const int cap = P.tab_cap, limit = cap * 3 / 4;
-  const int rmax = min(kVerifyThreads, limit / 3);  // matches per round: each adds at most three pairs
   {
     const double *src = P.pose + (size_t)blockIdx.x * kMaxHyp * 12;
     for (int i = tid; i < H * 12; i += kVerifyThreads) s_pose[i / 12][i % 12] = src[i];
   }
   if (tid < kMaxHyp) s_vote[tid] = 0;
-  int np = limit;  // pairs in the table (the same in every thread): "full" clears it for the first chunk
-  int tested = 0, nchunk = 0;
+  int nchunk = 0, span = kChunkMatches;
   unsigned long long cnt[kVotePlanes] = {};  // this lane's votes, bit-sliced
   int nadd = 0;                              // masks added since the last flush (the same in the whole warp)
-  // the vertices of match ce + tid, the next one this thread maps: loaded a round ahead, so that the
-  // loads (mostly from HBM: a keyframe's descriptors are read once per candidate) overlap the probing
-  float fa[9], fb[9];
-  if (tid < M) load_pair(P, q0, moff + tid, fa, fb);
   for (int cb = 0; cb < M; ++nchunk) {
-    if (limit - np < 3 * rmax) {  // no room for another round: start the table over
-      for (int i = tid; i < cap; i += kVerifyThreads) s_tag[i] = 0u;
-      if (tid == 0) s_npair = 0;
-      np = tested = 0;
+    const int cmax = min(M, cb + span);
+    for (int i = tid; i < cap; i += kVerifyThreads) s_tab[i] = 0u;
+    if (tid == 0) { s_npair = 0; s_stop = cmax; }
+    __syncthreads();
+    // ---- 1. pair ids of the chunk's matches: warp w maps matches cb + 32 w + kVerifyThreads i + lane.  A step
+    // is mapped while the vertices of the thread's next match and the match indices of the one after are in
+    // flight (mostly from HBM: a keyframe's descriptors are read once per candidate).
+    {
+      constexpr unsigned kAll = 0xffffffffu;
+      int j = cb + wid * 32 + lane;
+      DescVert x{}, y{};     // vertices of match j
+      uint32_t iq = 0, ig = 0;  // m_q / m_g of match j + kVerifyThreads
+      if (j < cmax) { x = P.qv[q0 + P.m_q[moff + j]]; y = P.dbv[P.m_g[moff + j]]; }
+      if (j + kVerifyThreads < cmax) { iq = P.m_q[moff + j + kVerifyThreads]; ig = P.m_g[moff + j + kVerifyThreads]; }
+      for (int base = cb + wid * 32; base < cmax; base += kVerifyThreads, j += kVerifyThreads) {
+        if (__any_sync(kAll, base >= *(volatile int *)&s_stop)) break;  // an earlier match already ends the chunk
+        const float4 v4[6] = {x.a, x.b, x.c, y.a, y.b, y.c};
+        if (j + kVerifyThreads < cmax) { x = P.qv[q0 + iq]; y = P.dbv[ig]; }
+        if (j + 2 * kVerifyThreads < cmax) { iq = P.m_q[moff + j + 2 * kVerifyThreads]; ig = P.m_g[moff + j + 2 * kVerifyThreads]; }
+        const bool act = j < cmax;
+        uint32_t key[3][6], h[3];
+        int id[3];
+        // most pairs are already in the table at their home position: look the three up at once
+#pragma unroll
+        for (int v = 0; v < 3; ++v) {
+#pragma unroll
+          for (int i = 0; i < 3; ++i) { key[v][i] = __float_as_uint((&v4[v].x)[i]); key[v][3 + i] = __float_as_uint((&v4[3 + v].x)[i]); }
+          h[v] = pair_hash(key[v]);
+          id[v] = act ? find_home(s_tab, s_key, key[v], h[v], cap) : -1;
+        }
+        bool fail = false;
+        uint32_t ids = 0u;
+#pragma unroll
+        for (int v = 0; v < 3; ++v) {
+          // the others probe on or insert: lanes holding the same pair agree first, so that one of them inserts it
+          const bool need = act && id[v] < 0;
+          if (__any_sync(kAll, need)) {
+            const int leader = __ffs(__match_any_sync(kAll, need ? h[v] : 0u)) - 1;  // 0 is no pair's hash
+            bool same = true;
+#pragma unroll
+            for (int i = 0; i < 6; ++i) same = (__shfl_sync(kAll, key[v][i], leader) == key[v][i]) && same;
+            const bool ins = need && (lane == leader || !same);
+            const int r = ins ? insert_pair(s_tab, s_key, &s_npair, key[v], h[v], cap, limit) : -1;
+            const int lid = __shfl_sync(kAll, r, leader);
+            if (need) id[v] = ins ? r : lid;
+          }
+          fail = fail || (act && id[v] < 0);
+          ids |= (uint32_t)id[v] << (10 * v);
+        }
+        if (act && !fail) s_ids[j - cb] = ids;
+        const unsigned bad = __ballot_sync(kAll, fail);
+        if (bad) {
+          if (lane == __ffs(bad) - 1) atomicMin(&s_stop, j);
+          break;
+        }
+      }
     }
     __syncthreads();
-    // ---- 1. pair ids of the chunk's matches
-    int ce = cb;
-    while (ce < M && ce - cb < kChunkMatches && limit - np >= 3 * rmax) {
-      const int r = min(rmax, min(M - ce, cb + kChunkMatches - ce));
-      uint32_t key[3][6], hsh[3];
-      int pos[3], pid[3] = {0, 0, 0}, st[3] = {0, 0, 0};  // st: 0 resolved, 1 probing, 2 same hash seen
-      if (tid < r) {
-#pragma unroll
-        for (int v = 0; v < 3; ++v) {
-#pragma unroll
-          for (int i = 0; i < 3; ++i) { key[v][i] = __float_as_uint(fa[v * 3 + i]); key[v][3 + i] = __float_as_uint(fb[v * 3 + i]); }
-          hsh[v] = pair_hash(key[v]);
-          pos[v] = hsh[v] & (cap - 1);
-          st[v] = 1;
-        }
-      }
-      if (ce + r + tid < M) load_pair(P, q0, moff + ce + r + tid, fa, fb);  // the next round starts at ce + r
-      for (;;) {
-        // claim an empty position or stop at one with the same hash.  A new pair's key is written by the
-        // thread that claimed it, so a same-hash position is compared only after the barrier.
-#pragma unroll
-        for (int v = 0; v < 3; ++v) {
-          while (st[v] == 1) {
-            uint32_t t = s_tag[pos[v]];
-            if (t == 0u) {
-              t = atomicCAS(&s_tag[pos[v]], 0u, hsh[v]);
-              if (t == 0u) {
-                const int u = atomicAdd(&s_npair, 1);
-                s_uid[pos[v]] = (uint16_t)u;
-#pragma unroll
-                for (int i = 0; i < 6; ++i) s_key[u][i] = key[v][i];
-                pid[v] = u; st[v] = 0;
-                break;
-              }
-            }
-            if (t == hsh[v]) st[v] = 2;
-            else pos[v] = (pos[v] + 1) & (cap - 1);
-          }
-        }
-        __syncthreads();
-        bool again = false;
-#pragma unroll
-        for (int v = 0; v < 3; ++v) {
-          if (st[v] == 2) {
-            const int u = s_uid[pos[v]];
-            bool eq = true;
-#pragma unroll
-            for (int i = 0; i < 6; ++i) eq = eq && s_key[u][i] == key[v][i];
-            if (eq) { pid[v] = u; st[v] = 0; }
-            else { pos[v] = (pos[v] + 1) & (cap - 1); st[v] = 1; again = true; }  // a hash collision: probe on
-          }
-        }
-        if (!__syncthreads_or(again)) break;
-      }
-      if (tid < r) s_ids[ce - cb + tid] = (uint32_t)pid[0] | (uint32_t)pid[1] << 10 | (uint32_t)pid[2] << 20;
-      np = s_npair;
-      ce += r;
-      __syncthreads();  // every thread has read s_npair before the next round adds to it
-    }
-    // ---- 2. outcomes of the pairs new to the table under every hypothesis
-    for (int u = tested + tid; u < np; u += kVerifyThreads) {
+    const int ce = s_stop, np = min(s_npair, limit);
+    span = ce == cb ? 1 : kChunkMatches;
+    // ---- 2. outcomes of the chunk's pairs under every hypothesis
+    for (int u = tid; u < np; u += kVerifyThreads) {
       const double px = __uint_as_float(s_key[u][0]), py = __uint_as_float(s_key[u][1]), pz = __uint_as_float(s_key[u][2]);
       const double bx = __uint_as_float(s_key[u][3]), by = __uint_as_float(s_key[u][4]), bz = __uint_as_float(s_key[u][5]);
       unsigned long long m = 0ull;
@@ -1959,7 +2016,6 @@ __global__ void __launch_bounds__(kVerifyThreads, 4) k_verify(VerifyParams P) {
       }
       s_hm[u] = m;
     }
-    tested = np;
     __syncthreads();
     // ---- 3. votes of the chunk's matches
     const int nc = ce - cb;

@@ -24,24 +24,24 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import orc  # noqa: E402
 from sgtd_b200 import synth  # noqa: E402
 
-PAIR_CAP, CHUNK_MATCHES, ROUND = 768, 2048, 128  # k_verify: kPairCap, kChunkMatches, matches per round
+PAIR_CAP, CHUNK_MATCHES = 768, 2048  # k_verify: kPairCap, kChunkMatches
 
 
-def chunks(qv, dv, M, cap=PAIR_CAP, chunk_matches=CHUNK_MATCHES, rnd=ROUND):
-    """chunks k_verify takes: rounds of up to `rnd` matches while the table has room for 3 new pairs per match
-    and the chunk holds fewer than chunk_matches matches; the table starts over when it is too full"""
-    rnd = min(rnd, cap // 3)
+def chunks(qv, dv, M, cap=PAIR_CAP, chunk_matches=CHUNK_MATCHES):
+    """chunks k_verify takes: a chunk ends at the first match whose new pairs do not fit the table, or after
+    chunk_matches matches, and the next one starts with an empty table.  Holes (ids reserved by racing inserts
+    of the same pair) can end a chunk earlier on the GPU; this counts none."""
     keys = np.concatenate([qv, dv], 1).reshape(M, 3, 6)
-    seen, n, j = set(), 0, 0
+    n, j = 0, 0
     while j < M:
         n += 1
-        if cap - len(seen) < 3 * rnd:
-            seen = set()
-        cb = j
-        while j < M and j - cb < chunk_matches and cap - len(seen) >= 3 * rnd:
-            for k in keys[j:j + min(rnd, M - j, cb + chunk_matches - j)].reshape(-1, 6):
-                seen.add(k.tobytes())
-            j = min(M, j + rnd, cb + chunk_matches)
+        seen, cb = set(), j
+        while j < M and j - cb < chunk_matches:
+            new = {k.tobytes() for k in keys[j]} - seen
+            if len(seen) + len(new) > cap:
+                break
+            seen |= new
+            j += 1
     return n
 
 
