@@ -238,6 +238,29 @@ int sgtd_frame_positions(sgtd_handle *h, const double *xyz, int64_t n);
 int sgtd_search_near(sgtd_handle *h, const sgtd_desc_batch *queries,
                      const double *prior_xyz, const double *radius,
                      sgtd_search_result **out);
+/* Loop-closure search: has this keyframe been here before?  Every descriptor of
+ * query scan q carries one frame id i_q, the scan's own keyframe id (from
+ * sgtd_build_descriptors with frame_ids, or sgtd_desc_batch_upload).  Query q
+ * votes only for keyframes f with f + skip_near_num < i_q (64-bit).  The result
+ * is what SearchLoop returns when keyframe i_q is searched against a database
+ * holding only keyframes [0, min(F, i_q - skip_near_num)), ids unchanged: the
+ * online loop, where keyframe i is searched before it is added and its last
+ * skip_near_num predecessors are excluded.  Pass config.skip_near_num.  Vote
+ * rows are 0 at every other keyframe; the sgtd_result_* calls and
+ * sgtd_gicp_refine_batch work on the result as usual.  A scan with no
+ * descriptors or a limit <= 0 gets no candidate and loop result (-1, 0).  A
+ * query carrying current_frame_id_ of the full database, with skip_near_num 0,
+ * gives exactly the result of sgtd_search.  In sgtd_result_stats, M counts the
+ * votes cast (all on allowed keyframes), E the bucket entries below each
+ * probe's cut (summed per probe), P the probes emitted (descriptors whose
+ * limit on this rank is 0 emit none); Q is the batch's.  Under options
+ * join_impl 0 / 2 (experimental joins without a loop form) the streaming
+ * vote kernel runs, as with vote_stream 1.  Collective on a handle with a
+ * communicator, like sgtd_search; the checks below come first on every rank.
+ * SGTD_E_INVALID for skip_near_num < 0, a scan whose descriptors carry more
+ * than one frame id, or NULL arguments. */
+int sgtd_search_loops(sgtd_handle *h, const sgtd_desc_batch *queries,
+                      int32_t skip_near_num, sgtd_search_result **out);
 int32_t sgtd_result_queries(const sgtd_search_result *r);
 /* loops: nq entries; cands: nq * candidate_num entries (entry c of query q at
  * q*candidate_num + c, valid for c < loops[q].ncand).  Either may be NULL. */

@@ -84,6 +84,7 @@ SYMBOLS = {
     "sgtd_search": (C.c_int, [_VP, _VP, C.POINTER(_VP)]),
     "sgtd_frame_positions": (C.c_int, [_VP, _VP, _I64]),
     "sgtd_search_near": (C.c_int, [_VP, _VP, _VP, _VP, C.POINTER(_VP)]),
+    "sgtd_search_loops": (C.c_int, [_VP, _VP, _I32, C.POINTER(_VP)]),
     "sgtd_result_queries": (_I32, [_VP]),
     "sgtd_result_download": (C.c_int, [_VP, _VP, _VP, _VP]),
     "sgtd_result_matches": (C.c_int, [_VP, _VP, _I32, _I32, _VP, _VP, _VP, _I64]),
@@ -483,6 +484,13 @@ class STDescManager:
         rad = np.ascontiguousarray(radius, np.float64).reshape(-1)
         out = C.c_void_p()
         self._chk(lib().sgtd_search_near(self._h, batch.ptr, _p(prior), _p(rad), C.byref(out)))
+        return SearchResult(self, out)
+
+    def search_loops(self, batch, skip):
+        """Loop-closure search: each scan of `batch` (whose descriptors carry its own keyframe id i) against
+        keyframes [0, i - skip) only.  Pass cfg.skip_near_num as `skip`."""
+        out = C.c_void_p()
+        self._chk(lib().sgtd_search_loops(self._h, batch.ptr, int(skip), C.byref(out)))
         return SearchResult(self, out)
 
     def db_fetch(self, g):

@@ -536,7 +536,23 @@ int sgtd_search_near(sgtd_handle *h, const sgtd_desc_batch *queries, const doubl
   else r = new sgtd_search_result();
   r->h = h;
   h->live_results.insert(r);
-  rc = search(h, queries, r, true);
+  rc = search(h, queries, r, SearchMode::Region);
+  if (rc) { cudaStreamSynchronize(h->stream); sgtd_result_free(r); return rc; }
+  *out = r;
+  return SGTD_OK;
+}
+
+int sgtd_search_loops(sgtd_handle *h, const sgtd_desc_batch *queries, int32_t skip_near_num, sgtd_search_result **out) {
+  if (!h || !queries || !out) SGTD_FAIL(h, SGTD_E_INVALID, "bad argument");
+  *out = nullptr;
+  if (skip_near_num < 0) SGTD_FAIL(h, SGTD_E_INVALID, "skip_near_num must be >= 0");
+  SetDevice sd(h->device);
+  sgtd_search_result *r;
+  if (!h->result_pool.empty()) { r = h->result_pool.back(); h->result_pool.pop_back(); }
+  else r = new sgtd_search_result();
+  r->h = h;
+  h->live_results.insert(r);
+  int rc = search(h, queries, r, SearchMode::Loops, skip_near_num);
   if (rc) { cudaStreamSynchronize(h->stream); sgtd_result_free(r); return rc; }
   *out = r;
   return SGTD_OK;

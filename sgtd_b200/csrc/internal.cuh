@@ -236,8 +236,11 @@ namespace sgtd {
 int build_descriptors(sgtd_handle *h, const sgtd_node *d_nodes, const std::vector<int64_t> &off,
                       const std::vector<uint32_t> &frame_ids, sgtd_desc_batch *out);
 int finalize_db(sgtd_handle *h);
-// region = true: sgtd_search_near, the queries' regions in h->region_q
-int search(sgtd_handle *h, const sgtd_desc_batch *q, sgtd_search_result *r, bool region = false);
+// which keyframes each query may vote for: every one (sgtd_search), those of its region (sgtd_search_near,
+// the queries' regions in h->region_q), or those more than loop_skip before its frame (sgtd_search_loops)
+enum class SearchMode { All, Region, Loops };
+int search(sgtd_handle *h, const sgtd_desc_batch *q, sgtd_search_result *r, SearchMode mode = SearchMode::All,
+           int64_t loop_skip = 0);
 void merge_topk_host(const int32_t *votes, const int32_t *frames, int nlists, int k,
                      int32_t *out_votes, int32_t *out_frames);
 }  // namespace sgtd

@@ -43,6 +43,7 @@ struct VoteParams {
   double rough;
   uint32_t *votes;         // nq * F
   unsigned long long *counters;  // Q,P,Pfound,E,M
+  const uint32_t *lim;     // loop-closure search: per descriptor, the local keyframes [0, lim) it may vote for
 };
 
 // Eigen evaluates a fixed-size reduction of three terms as e0 + (e1 + e2) (Redux.h, redux_novec_unroller
@@ -162,11 +163,22 @@ __device__ __forceinline__ bool table_find(const Bucket *table, uint64_t mask, u
 constexpr int kVoteThreads = 256;
 constexpr int kVoteUnroll = 4;
 
+// Loop-closure search: entries of a bucket are in keyframe order, so those a descriptor with limit `lim`
+// may vote for are a prefix of it.  Length of that prefix of the n local frame ids at fr.
+__device__ __forceinline__ uint32_t frames_below(const uint32_t *fr, uint32_t n, uint32_t lim) {
+  if (n == 0 || __ldg(fr + n - 1) < lim) return n;
+  uint32_t lo = 0, hi = n - 1;  // fr[hi] >= lim
+  while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (__ldg(fr + mid) < lim) lo = mid + 1; else hi = mid; }
+  return lo;
+}
+
 // One warp per query descriptor (persistent, strided).  Lanes 0..26 evaluate the
 // 27 probes and look their bucket up; the warp then streams every found bucket
 // with coalesced SoA loads (8 B x 3 + 4 B per entry) and votes with fire-and-
 // forget reductions (RED.ADD) into the query's per-keyframe counter row.
-template <bool kDoVote>
+// kLoop (sgtd_search_loops): a descriptor votes only for local keyframes below P.lim[d], streams each
+// bucket up to that cut, and emits no probe when its limit is 0.
+template <bool kDoVote, bool kLoop = false>
 __global__ void __launch_bounds__(kVoteThreads) k_vote(VoteParams P) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * kVoteThreads + threadIdx.x) >> 5;
@@ -179,7 +191,8 @@ __global__ void __launch_bounds__(kVoteThreads) k_vote(VoteParams P) {
     const double thr2 = a.thr2;
     const int qi = (int)a.qi;
     uint32_t off = 0, cnt = 0;
-    const bool pass = (a.mask >> lane) & 1u;
+    const uint32_t lim = kLoop ? P.lim[d] : 0u;
+    const bool pass = ((a.mask >> lane) & 1u) && (!kLoop || lim > 0);
     if (pass && !table_find(P.table, P.mask, probe_cell_key(r, lane), off, cnt)) cnt = 0;
     const unsigned m_pass = __ballot_sync(0xffffffffu, pass);
     unsigned m_found = __ballot_sync(0xffffffffu, cnt > 0);
@@ -189,7 +202,8 @@ __global__ void __launch_bounds__(kVoteThreads) k_vote(VoteParams P) {
       const int src = __ffs(m_found) - 1;
       m_found &= m_found - 1;
       const uint32_t o = __shfl_sync(0xffffffffu, off, src);
-      const uint32_t n = __shfl_sync(0xffffffffu, cnt, src);
+      uint32_t n = __shfl_sync(0xffffffffu, cnt, src);
+      if (kLoop) n = frames_below(P.fr + o, n, lim);
       cE += n;
       // kVoteUnroll x 32 entries per trip: all loads are issued before the first use so
       // that each warp keeps 4*kVoteUnroll independent 128/256-byte requests in flight.
@@ -207,8 +221,9 @@ __global__ void __launch_bounds__(kVoteThreads) k_vote(VoteParams P) {
         for (int u = 0; u < kVoteUnroll; ++u) {
           const uint32_t e = e0 + 32 * u + lane;
           const double d2 = sqn3(__dsub_rn(r.s[0], a[u]), __dsub_rn(r.s[1], b[u]), __dsub_rn(r.s[2], c[u]));
-          // (src.frame_id_ - db.frame_id_) > 0 on unsigned == "!=" (STDesc.cpp:373)
-          const bool hit = (e < n) && (f[u] + P.frame_lo != r.frame) && (d2 < thr2);
+          // (src.frame_id_ - db.frame_id_) > 0 on unsigned == "!=" (STDesc.cpp:373); loop mode: below the limit
+          const bool fok = kLoop ? f[u] < lim : f[u] + P.frame_lo != r.frame;
+          const bool hit = (e < n) && fok && (d2 < thr2);
           if (kDoVote && hit) atomicAdd(row + f[u], 1u);
           cM += __popc(__ballot_sync(0xffffffffu, hit));
         }
@@ -267,12 +282,15 @@ struct EmitParams2 {
   uint32_t *pkey, *pval;
   unsigned long long *cursor, *counters;
   uint32_t group_shift, group_div;  // sort key = (query / group_div) << group_shift | slot
+  const uint32_t *lim;              // loop-closure search: per descriptor limit (VoteParams::lim)
 };
 
 // A warp takes kEmitBatch consecutive descriptors per trip (lane = probe ordinal): the first table reads
 // of all of them are in flight together, and the output cursor -- one address for the whole grid -- is
 // advanced once per trip instead of once per descriptor.
+// kLoop: descriptors whose limit is 0 emit no probe, and E is left to the join (entries below each cut).
 constexpr int kEmitBatch = 4;
+template <bool kLoop = false>
 __global__ void __launch_bounds__(kVoteThreads, 4) k_probe_emit(EmitParams2 P) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * kVoteThreads + threadIdx.x) >> 5;
@@ -288,7 +306,7 @@ __global__ void __launch_bounds__(kVoteThreads, 4) k_probe_emit(EmitParams2 P) {
       const int64_t d = min(d0 + j, P.nd - 1);
       const DescRec r = P.q[d];
       const QAux a = P.aux[d];
-      pass[j] = (d0 + j < P.nd) && ((a.mask >> lane) & 1u);
+      pass[j] = (d0 + j < P.nd) && ((a.mask >> lane) & 1u) && (!kLoop || P.lim[d] > 0);
       grp[j] = (a.qi / P.group_div) << P.group_shift;
       key[j] = probe_cell_key(r, lane);
       pos[j] = mix64(key[j]) & P.mask;
@@ -315,7 +333,8 @@ __global__ void __launch_bounds__(kVoteThreads, 4) k_probe_emit(EmitParams2 P) {
       uint32_t esum = cnt[j];
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) esum += __shfl_xor_sync(0xffffffffu, esum, o);
-      cQ += (d0 + j < P.nd); cP += __popc(m_pass); cPf += __popc(m_found[j]); cE += esum;
+      cQ += (d0 + j < P.nd); cP += __popc(m_pass); cPf += __popc(m_found[j]);
+      if (!kLoop) cE += esum;
       total += __popc(m_found[j]);
     }
     unsigned long long base = 0;
@@ -354,6 +373,7 @@ struct JoinParams {
   const uint32_t *cut;             // parts > 1: per table slot, parts - 1 positions inside the bucket (first entry of part j + 1)
   int ngroups, parts;
   uint32_t group_shift;
+  const uint32_t *lim;             // loop-closure search: per descriptor limit (VoteParams::lim)
 };
 constexpr int kPlanMax = 32;  // query groups at most
 
@@ -445,12 +465,15 @@ __device__ __forceinline__ void red_inc_if_keep(uint32_t *addr, bool hit, uint64
 }
 
 static_assert(kVoteUnroll == 4, "k_vote_join pairs the entries of a trip as (0,1) and (2,3)");
-// kHint: REDs carry an L2 evict-last policy; kParts: passes over keyframe-range parts (option join_parts)
-template <bool kDoVote, bool kHint, bool kParts>
+// kHint: REDs carry an L2 evict-last policy; kParts: passes over keyframe-range parts (option join_parts);
+// kLoop (sgtd_search_loops): a probe votes only for local keyframes below its descriptor's limit, and a run
+// streams its bucket only up to the largest cut among its probes (entries are in keyframe order)
+template <bool kDoVote, bool kHint, bool kParts, bool kLoop = false>
 __global__ void __launch_bounds__(kVoteThreads, 5) k_vote_join(JoinParams P) {
   __shared__ double sh_s[kVoteThreads / 32][kJoinSeg][4];  // s0, s1, s2, thr2 of each probe of the segment (exact path)
   __shared__ float4 sh_f[kVoteThreads / 32][kJoinSeg];     // float s0, s1, s2, -thr2
-  __shared__ uint4 sh_g[kVoteThreads / 32][kJoinSeg];      // band half-width w (float bits), query frame id, vote row pointer
+  __shared__ uint4 sh_g[kVoteThreads / 32][kJoinSeg];      // band half-width w (float bits), query frame id (kLoop:
+                                                           // limit), vote row pointer
   __shared__ unsigned long long sh_plan[2 * (kPlanMax + 1)];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   if (kParts) {
@@ -463,6 +486,7 @@ __global__ void __launch_bounds__(kVoteThreads, 5) k_vote_join(JoinParams P) {
   uint64_t policy = 0;
   if (kHint) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(policy));
   uint32_t cM = 0;  // matches seen by this thread (only counted here when no votes are cast; else k_topk sums the rows)
+  unsigned long long cE = 0;  // kLoop: entries below the cut of this lane's probes
   while (true) {
     unsigned long long tk = 0;
     if (lane == 0) tk = atomicAdd(P.seg_counter, 1ull);
@@ -495,7 +519,7 @@ __global__ void __launch_bounds__(kVoteThreads, 5) k_vote_join(JoinParams P) {
       sh_f[wid][lane] = make_float4((float)r.s[0], (float)r.s[1], (float)r.s[2], -(float)a.thr2);
       const unsigned long long rowp = (unsigned long long)(P.votes + (size_t)a.qi * (size_t)P.F);
       // query frame id relative to this shard; (src.frame_id_ - db.frame_id_) > 0 on unsigned == "!=" (STDesc.cpp:373)
-      sh_g[wid][lane] = make_uint4(__float_as_uint(__double2float_ru(a.thr2 * P.band)), r.frame - P.frame_lo,
+      sh_g[wid][lane] = make_uint4(__float_as_uint(__double2float_ru(a.thr2 * P.band)), kLoop ? P.lim[d] : r.frame - P.frame_lo,
                                    (uint32_t)rowp, (uint32_t)(rowp >> 32));
     }
     __syncwarp();
@@ -506,11 +530,20 @@ __global__ void __launch_bounds__(kVoteThreads, 5) k_vote_join(JoinParams P) {
       const uint4 raw = __ldg(reinterpret_cast<const uint4 *>(&P.table[cur & P.slot_mask]));
       const uint32_t o = raw.z;
       uint32_t n = raw.w, e_lo = 0;  // this pass streams entries [e_lo, n) of the bucket: its keyframe part
+      uint32_t n_cut = n;
+      if (kLoop) {
+        // each probe of the run finds its own cut (counted once, in part 0); the run streams up to the largest
+        uint32_t c = 0;
+        if (lane >= i && lane < i + run) c = frames_below(P.fr + o, n, sh_g[wid][lane].y);
+        if (!kParts || part == 0) cE += c;
+        n_cut = __reduce_max_sync(0xffffffffu, c);
+      }
       if (kParts) {
         const uint32_t *c = P.cut + (size_t)(cur & P.slot_mask) * (uint32_t)(P.parts - 1);
         if (part > 0) e_lo = __ldg(c + part - 1);
         if (part < P.parts - 1) n = __ldg(c + part);
       }
+      if (kLoop) n = min(n, n_cut);  // a part wholly beyond the cut streams nothing
       for (uint32_t e0 = e_lo; e0 < n; e0 += 32 * kVoteUnroll) {
         float4 v[kVoteUnroll];
 #pragma unroll
@@ -548,7 +581,8 @@ __global__ void __launch_bounds__(kVoteThreads, 5) k_vote_join(JoinParams P) {
           }
 #pragma unroll
           for (int u = 0; u < kVoteUnroll; ++u) {
-            const bool hit = (fr[u] != g.y) && sd[u] < -wb;  // certainly a match
+            const bool fok = kLoop ? fr[u] < g.y : fr[u] != g.y;
+            const bool hit = fok && sd[u] < -wb;  // certainly a match
             if (kDoVote) { if (kHint) red_inc_if_keep(row + fr[u], hit, policy); else red_inc_if(row + fr[u], hit); }
             else cM += hit;
           }
@@ -557,7 +591,7 @@ __global__ void __launch_bounds__(kVoteThreads, 5) k_vote_join(JoinParams P) {
             uint32_t amb = 0;
 #pragma unroll
             for (int u = 0; u < kVoteUnroll; ++u)
-              if ((fr[u] != g.y) && fabsf(sd[u]) <= wb) amb |= 1u << u;
+              if ((kLoop ? fr[u] < g.y : fr[u] != g.y) && fabsf(sd[u]) <= wb) amb |= 1u << u;
             if (amb) cM += join_exact<kDoVote>(P.s0, P.s1, P.s2, P.fr, sh_s[wid][p], row, o, n, e0 + lane, amb);
           }
         }
@@ -570,6 +604,11 @@ __global__ void __launch_bounds__(kVoteThreads, 5) k_vote_join(JoinParams P) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) cM64 += __shfl_xor_sync(0xffffffffu, cM64, o);
     if (lane == 0 && cM64) atomicAdd(P.counters + 4, cM64);
+  }
+  if (kLoop) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) cE += __shfl_xor_sync(0xffffffffu, cE, o);
+    if (lane == 0 && cE) atomicAdd(P.counters + 3, cE);
   }
 }
 
@@ -1566,6 +1605,28 @@ __global__ void __launch_bounds__(kCollectThreads, kMinBlocks) k_collect_inv(Col
   }
 }
 
+// ============================ loop-closure search (sgtd_search_loops) ================
+// Scan q, whose descriptors all carry one frame id i_q, may only vote for keyframes f with f + skip < i_q:
+// the database [0, i_q - skip) of the online loop.  Entries of a bucket are in keyframe order, so the vote
+// kernels stream each bucket only up to the first entry at or beyond the limit, and the vote rows are those
+// of a database holding that prefix (votes depend on each keyframe's own descriptors only).
+// One CTA per scan: the limit of each descriptor on this rank, clamp(frame - skip - frame_lo, 0, F), and a
+// flag for a scan whose descriptors carry more than one frame id.
+__global__ void k_loop_limits(const DescRec *q, const int64_t *q_off, int64_t skip, int64_t frame_lo, int64_t F,
+                              uint32_t *lim, uint32_t *mixed) {
+  const int64_t d0 = q_off[blockIdx.x], d1 = q_off[blockIdx.x + 1];
+  if (d0 >= d1) return;
+  const uint32_t f0 = q[d0].frame;
+  bool bad = false;
+  for (int64_t d = d0 + threadIdx.x; d < d1; d += blockDim.x) {
+    const uint32_t f = q[d].frame;
+    bad |= f != f0;
+    const int64_t l = (int64_t)f - skip - frame_lo;
+    lim[d] = (uint32_t)(l <= 0 ? 0 : (l < F ? l : F));
+  }
+  if (__syncthreads_or(bad) && threadIdx.x == 0) *mixed = 1u;
+}
+
 // ============================ region search (sgtd_search_near) =======================
 // A query q may only vote for the keyframes f of its region: f has a position p (sgtd_frame_positions) and
 // (dx*dx + dy*dy) + dz*dz <= r*r with d = p - c_q, in double without contraction.  Votes depend on each
@@ -2166,7 +2227,8 @@ static float ev_ms(cudaEvent_t a, cudaEvent_t b) { float ms = 0; cudaEventElapse
 // keyframes, summed over the batch, are below this share of (queries x entries on this rank).
 constexpr double kRegionSparseShare = 0.0015;
 
-int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, bool region) {
+int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, SearchMode mode, int64_t loop_skip) {
+  const bool region = mode == SearchMode::Region, loops = mode == SearchMode::Loops;
   cudaStream_t st = h->stream;
   int rc = finalize_db(h);
   if (rc) return rc;
@@ -2203,7 +2265,9 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
   size_t o_aux = o; o += al((size_t)std::max<int64_t>(qb->n, 1) * sizeof(QAux));
   // vote formulation: bucket-major join (default) or per-probe streaming (SGTD_VOTE_MODE=stream)
   bool m_by_topk = false;  // the join leaves the match count (stats) to k_topk
-  const bool join_mode = !h->opt.vote_stream && qb->n > 0 && h->rec.n > 0;
+  // The experimental joins (join_impl 0 / 2) have no loop-closure form, and their index holds no 16-byte
+  // entries for the default join: a loop search under them runs the streaming kernel.
+  const bool join_mode = !h->opt.vote_stream && qb->n > 0 && h->rec.n > 0 && !(loops && h->opt.join_impl != 1);
   bool join_timed = false;
   const bool sort_q = !join_mode && qb->n > 0;  // streaming mode walks descriptors in cell-key order (L2 reuse)
   size_t cubj = 0;
@@ -2245,6 +2309,9 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
   size_t o_roff = o; o += region_votes ? al((size_t)(nq + 1) * 8) : 0;
   size_t o_rent = o; o += region_votes ? al(8) : 0;
   size_t o_rcub = o; o += region_votes ? al(cubr) : 0;
+  // loop-closure search: per-descriptor limits, the mixed-frame flag
+  size_t o_lim = o; o += loops ? al((size_t)std::max<int64_t>(qb->n, 1) * 4) : 0;
+  size_t o_mixed = o; o += loops ? al(4) : 0;
   SGTD_CUDA(h, h->scratch.reserve(o, st, false));
   unsigned char *S = h->scratch.p;
   int32_t *lv = (int32_t *)(S + o_lv), *lf = (int32_t *)(S + o_lf), *gv = (int32_t *)(S + o_gv);
@@ -2255,6 +2322,17 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
   // half-width of the FP32 decision band of the join's pre-filter, relative to thr^2 (see k_vote_join)
   const double join_band = 2.5e-6 * (1.0 + 1.0 / h->c.rough);
   SGTD_CUDA(h, cudaEventRecord(ev[0], st));
+  const uint32_t *d_lim = loops ? (const uint32_t *)(S + o_lim) : nullptr;
+  if (loops && qb->n > 0) {
+    // limits and validation before any collective: every rank sees the same queries, so every rank fails alike
+    uint32_t *d_mixed = (uint32_t *)(S + o_mixed), mixed = 0;
+    SGTD_CUDA(h, cudaMemsetAsync(d_mixed, 0, 4, st));
+    k_loop_limits<<<nq, 256, 0, st>>>(qb->rec.p, qb->d_off.p, loop_skip, h->frame_lo(), F, (uint32_t *)(S + o_lim), d_mixed);
+    SGTD_LAUNCHED(h);
+    SGTD_CUDA(h, cudaMemcpyAsync(&mixed, d_mixed, 4, cudaMemcpyDeviceToHost, st));
+    SGTD_CUDA(h, cudaStreamSynchronize(st));
+    if (mixed) SGTD_FAIL(h, SGTD_E_INVALID, "a query scan's descriptors carry more than one frame id");
+  }
   if (qb->n > 0) {
     SGTD_CUDA(h, cudaMemsetAsync(S + o_qpr, 0, (size_t)nq * 4, st));
     k_qaux<<<(unsigned)((qb->n + 255) / 256), 256, 0, st>>>(qb->rec.p, qb->d_off.p, nq, qb->n, h->c.rough, aux,
@@ -2325,11 +2403,13 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
     V.table = h->table.p; V.mask = h->table_mask;
     V.s0 = h->v_s0.p; V.s1 = h->v_s1.p; V.s2 = h->v_s2.p; V.fr = h->v_frame.p;
     V.frame_lo = (uint32_t)h->frame_lo(); V.F = Fa; V.rough = h->c.rough;
-    V.votes = r->votes.p; V.counters = r->counters.p;
+    V.votes = r->votes.p; V.counters = r->counters.p; V.lim = d_lim;
     const int64_t warps_needed = qb->n;
     int grid = (int)std::min<int64_t>((warps_needed * 32 + kVoteThreads - 1) / kVoteThreads, (int64_t)h->sm_count * 8);
     if (!join_mode) {
-      if (h->opt.debug_novote) k_vote<false><<<grid, kVoteThreads, 0, st>>>(V);
+      if (loops && h->opt.debug_novote) k_vote<false, true><<<grid, kVoteThreads, 0, st>>>(V);
+      else if (loops) k_vote<true, true><<<grid, kVoteThreads, 0, st>>>(V);
+      else if (h->opt.debug_novote) k_vote<false><<<grid, kVoteThreads, 0, st>>>(V);
       else k_vote<true><<<grid, kVoteThreads, 0, st>>>(V);
       SGTD_LAUNCHED(h);
       SGTD_CUDA(h, cudaGetLastError());
@@ -2339,7 +2419,7 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
       EmitParams2 E2{};
       E2.q = qb->rec.p; E2.aux = aux; E2.nd = qb->n; E2.table = h->table.p; E2.mask = h->table_mask;
       E2.pkey = (uint32_t *)(S + o_jk0); E2.pval = (uint32_t *)(S + o_jv0);
-      E2.cursor = d_cursor; E2.counters = r->counters.p;
+      E2.cursor = d_cursor; E2.counters = r->counters.p; E2.lim = d_lim;
       int sbits = 1;
       while ((1ull << sbits) <= h->table_mask) ++sbits;
       // Probes are processed query-group by query-group so that the vote rows being reduced into
@@ -2356,7 +2436,8 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
       ngroups = (nq + (int)E2.group_div - 1) / (int)E2.group_div;  // groups that exist
       int gbits = 0;
       while ((1 << gbits) < ngroups) ++gbits;
-      k_probe_emit<<<grid, kVoteThreads, 0, st>>>(E2);
+      if (loops) k_probe_emit<true><<<grid, kVoteThreads, 0, st>>>(E2);
+      else k_probe_emit<<<grid, kVoteThreads, 0, st>>>(E2);
       SGTD_LAUNCHED(h);
       unsigned long long npairs = 0;
       SGTD_CUDA(h, cudaMemcpyAsync(&npairs, d_cursor, 8, cudaMemcpyDeviceToHost, st));
@@ -2375,6 +2456,7 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
         J.frame_lo = (uint32_t)h->frame_lo(); J.F = Fa; J.votes = r->votes.p;
         J.seg_counter = d_cursor + 1; J.counters = r->counters.p; J.slot_mask = (uint32_t)((1ull << sbits) - 1);
         J.plan = (unsigned long long *)(S + o_plan); J.ngroups = ngroups; J.parts = parts; J.group_shift = (uint32_t)sbits;
+        J.lim = d_lim;
         if (!run_join && parts > 1) {
           if (h->v_cut_parts != parts) {
             const uint64_t nslots = h->table_mask + 1;
@@ -2399,7 +2481,14 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, boo
         }
         if (!run_join) {
           SGTD_CUDA(h, cudaEventRecord(ev[8], st));
-          if (h->opt.debug_novote) k_vote_join<false, false, false><<<jgrid, kVoteThreads, 0, st>>>(J);
+          if (loops) {
+            if (h->opt.debug_novote) k_vote_join<false, false, false, true><<<jgrid, kVoteThreads, 0, st>>>(J);
+            else if (parts > 1 && h->opt.join_hint) k_vote_join<true, true, true, true><<<jgrid, kVoteThreads, 0, st>>>(J);
+            else if (parts > 1) k_vote_join<true, false, true, true><<<jgrid, kVoteThreads, 0, st>>>(J);
+            else if (h->opt.join_hint) k_vote_join<true, true, false, true><<<jgrid, kVoteThreads, 0, st>>>(J);
+            else k_vote_join<true, false, false, true><<<jgrid, kVoteThreads, 0, st>>>(J);
+            m_by_topk = !h->opt.debug_novote;
+          } else if (h->opt.debug_novote) k_vote_join<false, false, false><<<jgrid, kVoteThreads, 0, st>>>(J);
           else if (parts > 1 && h->opt.join_hint) { k_vote_join<true, true, true><<<jgrid, kVoteThreads, 0, st>>>(J); m_by_topk = true; }
           else if (parts > 1) { k_vote_join<true, false, true><<<jgrid, kVoteThreads, 0, st>>>(J); m_by_topk = true; }
           else if (h->opt.join_hint) { k_vote_join<true, true, false><<<jgrid, kVoteThreads, 0, st>>>(J); m_by_topk = true; }
