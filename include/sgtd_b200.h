@@ -261,6 +261,32 @@ int sgtd_search_near(sgtd_handle *h, const sgtd_desc_batch *queries,
  * than one frame id, or NULL arguments. */
 int sgtd_search_loops(sgtd_handle *h, const sgtd_desc_batch *queries,
                       int32_t skip_near_num, sgtd_search_result **out);
+/* Range search: query q votes only for the keyframes in the union of its
+ * ranges of global keyframe ids, the half-open intervals [ranges[2j],
+ * ranges[2j+1]) for j in [range_off[q], range_off[q+1]) (range_off: nq + 1
+ * entries).  The result is what SearchLoop returns against a database holding
+ * only those keyframes, ids unchanged: votes, ranking, match and inlier
+ * lists, poses and the loop result; vote rows are 0 at every other keyframe.
+ * A descriptor still never votes for its own frame id, as in sgtd_search.  A
+ * query without ranges, or without an allowed keyframe, gets no candidate and
+ * loop result (-1, 0).  hi beyond the database is clipped: [0, INT64_MAX)
+ * allows every keyframe.  Prefixes (loop closure with any extra rule), one
+ * recording of a multi-session map or everything but it, or the runs of ids
+ * of keyframes within a distance of a trajectory point are all short range
+ * lists.  Both arrays may be host or device pointers and are consumed before
+ * the call returns.  The vote formulation is chosen as for sgtd_search_near
+ * (option region_vote forces one), and sgtd_result_stats follows its rules:
+ * M counts the votes cast on allowed keyframes, Q and P are the batch's, E
+ * and Pfound depend on the formulation that ran.  The sgtd_result_* calls and
+ * sgtd_gicp_refine_batch work on the result as usual.  Collective on a handle
+ * with a communicator, like sgtd_search; the checks below come first on every
+ * rank.  SGTD_E_INVALID for range_off[0] != 0, a decreasing range_off, a range
+ * without 0 <= lo < hi, a query's ranges not ascending and disjoint
+ * (hi_j <= lo_{j+1}; touching ranges are fine), or NULL arguments (ranges may
+ * be NULL when nq == 0). */
+int sgtd_search_ranges(sgtd_handle *h, const sgtd_desc_batch *queries,
+                       const int64_t *ranges, const int64_t *range_off,
+                       sgtd_search_result **out);
 int32_t sgtd_result_queries(const sgtd_search_result *r);
 /* loops: nq entries; cands: nq * candidate_num entries (entry c of query q at
  * q*candidate_num + c, valid for c < loops[q].ncand).  Either may be NULL. */

@@ -85,6 +85,7 @@ SYMBOLS = {
     "sgtd_frame_positions": (C.c_int, [_VP, _VP, _I64]),
     "sgtd_search_near": (C.c_int, [_VP, _VP, _VP, _VP, C.POINTER(_VP)]),
     "sgtd_search_loops": (C.c_int, [_VP, _VP, _I32, C.POINTER(_VP)]),
+    "sgtd_search_ranges": (C.c_int, [_VP, _VP, _VP, _VP, C.POINTER(_VP)]),
     "sgtd_result_queries": (_I32, [_VP]),
     "sgtd_result_download": (C.c_int, [_VP, _VP, _VP, _VP]),
     "sgtd_result_matches": (C.c_int, [_VP, _VP, _I32, _I32, _VP, _VP, _VP, _I64]),
@@ -180,6 +181,34 @@ def merge_topk_host(votes, frames, k):
     if rc:
         raise SgtdError(rc, "sgtd_merge_topk_host")
     return ov, of
+
+
+def ball_ranges(positions, centers, radius, limits=None, chunk=64):
+    """Keyframe-id ranges for sgtd_search_ranges: for each center q, the runs of consecutive ids f whose
+    position lies within radius[q] of centers[q] -- (dx*dx + dy*dy) + dz*dz <= r*r in double, the test of
+    sgtd_search_near -- and, with `limits`, f < limits[q] as well (loop closure: limits[q] = i_q - skip).
+    positions: float64 [F, 3]; centers: [nq, 3]; radius and limits: scalars or [nq].
+    Returns (ranges int64 [R, 2], offsets int64 [nq + 1])."""
+    pos = np.asarray(positions, np.float64).reshape(-1, 3)
+    cen = np.asarray(centers, np.float64).reshape(-1, 3)
+    nq, nf = cen.shape[0], pos.shape[0]
+    r = np.broadcast_to(np.asarray(radius, np.float64), (nq,))
+    lim = None if limits is None else np.broadcast_to(np.asarray(limits, np.int64), (nq,))
+    ids = np.arange(nf)
+    runs, counts = [], np.zeros(nq, np.int64)
+    for q0 in range(0, nq, chunk):
+        q1 = min(nq, q0 + chunk)
+        d = pos[None, :, :] - cen[q0:q1, None, :]
+        ok = ((d[..., 0] * d[..., 0] + d[..., 1] * d[..., 1]) + d[..., 2] * d[..., 2]) <= (r[q0:q1] * r[q0:q1])[:, None]
+        if lim is not None:
+            ok &= ids[None, :] < lim[q0:q1, None]
+        step = np.diff(np.pad(ok, ((0, 0), (1, 1))).astype(np.int8), axis=1)
+        sq, lo = np.nonzero(step == 1)      # row-major: per query, ascending
+        _, hi = np.nonzero(step == -1)
+        runs.append(np.column_stack([lo, hi]))
+        counts[q0:q1] = np.bincount(sq, minlength=q1 - q0)
+    ranges = np.concatenate(runs).astype(np.int64) if runs else np.zeros((0, 2), np.int64)
+    return ranges.reshape(-1, 2), np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
 
 
 def db_key(desc, cfg=None):
@@ -491,6 +520,18 @@ class STDescManager:
         keyframes [0, i - skip) only.  Pass cfg.skip_near_num as `skip`."""
         out = C.c_void_p()
         self._chk(lib().sgtd_search_loops(self._h, batch.ptr, int(skip), C.byref(out)))
+        return SearchResult(self, out)
+
+    def search_ranges(self, batch, ranges, offsets):
+        """search() with query q restricted to the keyframes in its ranges [lo, hi) of global ids:
+        ranges[offsets[q]:offsets[q + 1]] (int64 [R, 2], [nq + 1]; host arrays, or raw device pointers).
+        See ball_ranges for the runs of ids near a position."""
+        if ranges is not None and not isinstance(ranges, int):
+            ranges = np.ascontiguousarray(ranges, np.int64).reshape(-1, 2)
+        if offsets is not None and not isinstance(offsets, int):
+            offsets = np.ascontiguousarray(offsets, np.int64).reshape(-1)
+        out = C.c_void_p()
+        self._chk(lib().sgtd_search_ranges(self._h, batch.ptr, _p(ranges), _p(offsets), C.byref(out)))
         return SearchResult(self, out)
 
     def db_fetch(self, g):

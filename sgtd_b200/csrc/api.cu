@@ -108,6 +108,16 @@ static void destroy_batch(sgtd_desc_batch *b) { release_batch(b); delete b; }
 static void destroy_result(sgtd_search_result *r) { release_result(r); delete r; }
 constexpr size_t kPoolMax = 4;
 
+// host copy of n values the caller passed as a host or device pointer
+template <class T>
+static int fetch_host(sgtd_handle *h, const T *src, size_t n, std::vector<T> &out) {
+  out.resize(n);
+  if (n == 0) return SGTD_OK;
+  if (is_device_ptr(src)) SGTD_CUDA(h, cudaMemcpy(out.data(), src, n * sizeof(T), cudaMemcpyDeviceToHost));
+  else memcpy(out.data(), src, n * sizeof(T));
+  return SGTD_OK;
+}
+
 extern "C" {
 
 int sgtd_abi_version(void) { return SGTD_ABI_VERSION; }
@@ -264,7 +274,7 @@ int sgtd_destroy(sgtd_handle *h) {
   h->rec.release(); h->vert.release(); h->d_frame_off.release();
   h->v_s0.release(); h->v_s1.release(); h->v_s2.release(); h->v_frame.release(); h->v_pack.release(); h->v_pack8.release();
   h->table.release(); h->v_cut.release(); h->f_key.release(); h->f_g.release(); h->f_side.release(); h->scratch.release(); h->stage_in.release(); h->uniq_bitmap.release();
-  h->pos.release(); h->region_q.release(); h->region_items.release();
+  h->pos.release(); h->region_q.release(); h->region_items.release(); h->range_q.release();
   if (h->s1pool && h->s1pool_free) h->s1pool_free(h->s1pool);
   if (h->gicp_pool && h->gicp_pool_free) h->gicp_pool_free(h->gicp_pool);
   for (auto *r : h->result_pool) destroy_result(r);
@@ -478,20 +488,11 @@ int sgtd_search(sgtd_handle *h, const sgtd_desc_batch *queries, sgtd_search_resu
   return SGTD_OK;
 }
 
-// host copy of n doubles the caller passed as a host or device pointer
-static int fetch_doubles(sgtd_handle *h, const double *src, size_t n, std::vector<double> &out) {
-  out.resize(n);
-  if (n == 0) return SGTD_OK;
-  if (is_device_ptr(src)) SGTD_CUDA(h, cudaMemcpy(out.data(), src, n * 8, cudaMemcpyDeviceToHost));
-  else memcpy(out.data(), src, n * 8);
-  return SGTD_OK;
-}
-
 int sgtd_frame_positions(sgtd_handle *h, const double *xyz, int64_t n) {
   if (!h || n < 0 || (n > 0 && !xyz)) SGTD_FAIL(h, SGTD_E_INVALID, "bad argument");
   SetDevice sd(h->device);
   std::vector<double> p;
-  int rc = fetch_doubles(h, xyz, (size_t)n * 3, p);
+  int rc = fetch_host(h, xyz, (size_t)n * 3, p);
   if (rc) return rc;
   for (double v : p)
     if (!std::isfinite(v)) SGTD_FAIL(h, SGTD_E_INVALID, "non-finite keyframe position");
@@ -517,8 +518,8 @@ int sgtd_search_near(sgtd_handle *h, const sgtd_desc_batch *queries, const doubl
   if (!h->pos_set) SGTD_FAIL(h, SGTD_E_INVALID, "no keyframe positions set (sgtd_frame_positions)");
   SetDevice sd(h->device);
   std::vector<double> c, rad;
-  int rc = fetch_doubles(h, prior_xyz, (size_t)nq * 3, c);
-  if (!rc) rc = fetch_doubles(h, radius, (size_t)nq, rad);
+  int rc = fetch_host(h, prior_xyz, (size_t)nq * 3, c);
+  if (!rc) rc = fetch_host(h, radius, (size_t)nq, rad);
   if (rc) return rc;
   std::vector<double> reg((size_t)std::max(nq, 1) * 4);
   for (int q = 0; q < nq; ++q) {
@@ -553,6 +554,42 @@ int sgtd_search_loops(sgtd_handle *h, const sgtd_desc_batch *queries, int32_t sk
   r->h = h;
   h->live_results.insert(r);
   int rc = search(h, queries, r, SearchMode::Loops, skip_near_num);
+  if (rc) { cudaStreamSynchronize(h->stream); sgtd_result_free(r); return rc; }
+  *out = r;
+  return SGTD_OK;
+}
+
+int sgtd_search_ranges(sgtd_handle *h, const sgtd_desc_batch *queries, const int64_t *ranges, const int64_t *range_off,
+                       sgtd_search_result **out) {
+  if (!h || !queries || !range_off || !out) SGTD_FAIL(h, SGTD_E_INVALID, "bad argument");
+  *out = nullptr;
+  const int nq = queries->nscans;
+  if (nq > 0 && !ranges) SGTD_FAIL(h, SGTD_E_INVALID, "bad argument");
+  SetDevice sd(h->device);
+  // validated on the host before any collective: every rank sees the same arguments, so every rank fails alike
+  std::vector<int64_t> off, rg;
+  int rc = fetch_host(h, range_off, (size_t)nq + 1, off);
+  if (rc) return rc;
+  if (off[0] != 0) SGTD_FAIL(h, SGTD_E_INVALID, "range_off[0] must be 0");
+  for (int q = 0; q < nq; ++q)
+    if (off[q + 1] < off[q]) SGTD_FAIL(h, SGTD_E_INVALID, "range_off must be non-decreasing");
+  const int64_t nr = off[nq];
+  if (nr > 0 && (rc = fetch_host(h, ranges, (size_t)nr * 2, rg))) return rc;
+  for (int q = 0; q < nq; ++q)
+    for (int64_t j = off[q]; j < off[q + 1]; ++j) {
+      const int64_t lo = rg[2 * j], hi = rg[2 * j + 1];
+      if (lo < 0 || lo >= hi) SGTD_FAIL(h, SGTD_E_INVALID, "every range [lo, hi) needs 0 <= lo < hi");
+      if (j > off[q] && lo < rg[2 * j - 1]) SGTD_FAIL(h, SGTD_E_INVALID, "a query's ranges must be ascending and disjoint");
+    }
+  off.insert(off.end(), rg.begin(), rg.end());
+  SGTD_CUDA(h, h->range_q.reserve(off.size(), h->stream, false));
+  SGTD_CUDA(h, cudaMemcpyAsync(h->range_q.p, off.data(), off.size() * 8, cudaMemcpyHostToDevice, h->stream));
+  sgtd_search_result *r;
+  if (!h->result_pool.empty()) { r = h->result_pool.back(); h->result_pool.pop_back(); }
+  else r = new sgtd_search_result();
+  r->h = h;
+  h->live_results.insert(r);
+  rc = search(h, queries, r, SearchMode::Ranges);
   if (rc) { cudaStreamSynchronize(h->stream); sgtd_result_free(r); return rc; }
   *out = r;
   return SGTD_OK;

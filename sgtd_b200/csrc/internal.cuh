@@ -199,7 +199,9 @@ struct sgtd_handle {
   int64_t n_pos = 0;
   bool pos_set = false;
   sgtd::DevBuf<double> region_q;        // sgtd_search_near: {cx, cy, cz, r} per query of the running call
-  sgtd::DevBuf<uint32_t> region_items;  // sgtd_search_near: allowed keyframes of every query (sparse vote)
+  sgtd::DevBuf<uint32_t> region_items;  // sgtd_search_near / _ranges: allowed keyframes of every query (sparse vote)
+  // sgtd_search_ranges: the running call's range_off (nq + 1) then its ranges (2 per range), global ids
+  sgtd::DevBuf<int64_t> range_q;
   // scratch + recycled objects: steady-state build/search calls do no cudaMalloc/cudaFree
   sgtd::DevBuf<uint32_t> uniq_bitmap;
   sgtd::DevBuf<unsigned char> scratch;
@@ -237,8 +239,9 @@ int build_descriptors(sgtd_handle *h, const sgtd_node *d_nodes, const std::vecto
                       const std::vector<uint32_t> &frame_ids, sgtd_desc_batch *out);
 int finalize_db(sgtd_handle *h);
 // which keyframes each query may vote for: every one (sgtd_search), those of its region (sgtd_search_near,
-// the queries' regions in h->region_q), or those more than loop_skip before its frame (sgtd_search_loops)
-enum class SearchMode { All, Region, Loops };
+// the queries' regions in h->region_q), those more than loop_skip before its frame (sgtd_search_loops), or
+// those in its keyframe-id ranges (sgtd_search_ranges, the ranges in h->range_q)
+enum class SearchMode { All, Region, Loops, Ranges };
 int search(sgtd_handle *h, const sgtd_desc_batch *q, sgtd_search_result *r, SearchMode mode = SearchMode::All,
            int64_t loop_skip = 0);
 void merge_topk_host(const int32_t *votes, const int32_t *frames, int nlists, int k,

@@ -1750,6 +1750,105 @@ __global__ void __launch_bounds__(kRegionThreads) k_region_vote(const uint32_t *
   if (lane == 0 && cE) atomicAdd(counters + 3, cE);
 }
 
+// ============================ range search (sgtd_search_ranges) ======================
+// Query q may only vote for the keyframes in the union of its ranges [lo, hi) of global ids, ascending and
+// disjoint (checked on the host): rng[2j], rng[2j + 1] for j in [roff[q], roff[q + 1]).  The vote rows with
+// every other entry at zero are those of a database holding only those keyframes, as for region search, and
+// the two vote formulations are region search's with these allowed sets.
+
+// [lo, hi) clipped to this rank's keyframes, in local ids: [*a, *b), empty when *a == *b
+__device__ __forceinline__ void range_local(const int64_t *rng, int64_t j, int64_t frame_lo, int64_t F, int64_t *a,
+                                            int64_t *b) {
+  const int64_t lo = rng[2 * j] - frame_lo, hi = rng[2 * j + 1] - frame_lo;
+  *a = lo < 0 ? 0 : (lo < F ? lo : F);
+  *b = hi < *a ? *a : (hi < F ? hi : F);
+}
+
+// One CTA per query: allowed keyframes of this rank (cnt[q]) and the vote-index entries they hold (summed into
+// *entries), both from the clipped range ends: O(ranges), not O(F).
+__global__ void __launch_bounds__(kRegionThreads) k_ranges_count(const int64_t *roff, const int64_t *rng, int64_t frame_lo,
+                                                                 int64_t F, const int64_t *frame_off, int64_t *cnt,
+                                                                 unsigned long long *entries) {
+  __shared__ unsigned long long s_sum[2][kRegionThreads / 32];
+  const int q = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  unsigned long long n = 0, e = 0;
+  for (int64_t j = roff[q] + threadIdx.x; j < roff[q + 1]; j += kRegionThreads) {
+    int64_t a, b;
+    range_local(rng, j, frame_lo, F, &a, &b);
+    n += (unsigned long long)(b - a);
+    e += (unsigned long long)(frame_off[b] - frame_off[a]);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) { n += __shfl_xor_sync(0xffffffffu, n, o); e += __shfl_xor_sync(0xffffffffu, e, o); }
+  if (lane == 0) { s_sum[0][wid] = n; s_sum[1][wid] = e; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long tn = 0, te = 0;
+    for (int w = 0; w < kRegionThreads / 32; ++w) { tn += s_sum[0][w]; te += s_sum[1][w]; }
+    cnt[q] = (int64_t)tn;
+    if (te) atomicAdd(entries, te);
+  }
+}
+
+// One CTA per query: its allowed keyframes in ascending order at items[off[q] ..), and the Q / P statistics of
+// the query (as k_region_fill).  Ranges go in chunks of one per thread: a block scan of their clipped lengths
+// gives each range's first item, then the block writes the chunk's items evenly, each thread finding the
+// range of its item by binary search over the chunk's starts.
+__global__ void __launch_bounds__(kRegionThreads) k_ranges_fill(const int64_t *roff, const int64_t *rng, int64_t frame_lo,
+                                                                int64_t F, const int64_t *off, uint32_t *items,
+                                                                const int64_t *q_off, const uint32_t *qprobes,
+                                                                unsigned long long *counters) {
+  __shared__ uint32_t s_start[kRegionThreads], s_a[kRegionThreads], s_warp[kRegionThreads / 32];
+  const int q = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  int64_t base = off[q];
+  for (int64_t j0 = roff[q]; j0 < roff[q + 1]; j0 += kRegionThreads) {
+    const int64_t j = j0 + threadIdx.x;
+    int64_t a = 0, b = 0;
+    if (j < roff[q + 1]) range_local(rng, j, frame_lo, F, &a, &b);
+    const uint32_t len = (uint32_t)(b - a);  // within [0, F), F < 2^32: so are the sums below
+    uint32_t incl = len;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += v;
+    }
+    if (lane == 31) s_warp[wid] = incl;
+    __syncthreads();
+    uint32_t before = 0, total = 0;
+#pragma unroll
+    for (int w = 0; w < kRegionThreads / 32; ++w) { before += w < wid ? s_warp[w] : 0u; total += s_warp[w]; }
+    s_start[threadIdx.x] = before + incl - len;
+    s_a[threadIdx.x] = (uint32_t)a;
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < total; i += kRegionThreads) {
+      int lo = 0, hi = kRegionThreads - 1;  // the range of item i: last t with s_start[t] <= i (it has len > 0)
+      while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (s_start[mid] <= i) lo = mid; else hi = mid - 1; }
+      items[base + i] = s_a[lo] + (i - s_start[lo]);
+    }
+    base += total;
+    __syncthreads();  // s_warp, s_start and s_a are rewritten by the next chunk
+  }
+  if (threadIdx.x == 0) {
+    atomicAdd(counters + 0, (unsigned long long)(q_off[q + 1] - q_off[q]));
+    atomicAdd(counters + 1, (unsigned long long)qprobes[q]);
+  }
+}
+
+// Dense formulation: after the unrestricted vote, every entry of a keyframe outside the query's ranges set to
+// zero.  Each keyframe finds the last range with lo <= its id by binary search: O(F log ranges) per query.
+__global__ void __launch_bounds__(kRegionThreads) k_ranges_mask(const int64_t *roff, const int64_t *rng, int64_t frame_lo,
+                                                                int64_t F, uint32_t *votes) {
+  const int q = blockIdx.x;
+  const int64_t r0 = roff[q], r1 = roff[q + 1];
+  uint32_t *row = votes + (size_t)q * (size_t)F;
+  for (int64_t f = (int64_t)blockIdx.y * kRegionThreads + threadIdx.x; f < F; f += (int64_t)gridDim.y * kRegionThreads) {
+    const int64_t g = frame_lo + f;
+    int64_t lo = r0, hi = r1;  // first range with lo > g, over [r0, r1)
+    while (lo < hi) { const int64_t mid = (lo + hi) >> 1; if (rng[2 * mid] <= g) lo = mid + 1; else hi = mid; }
+    if (lo == r0 || g >= rng[2 * (lo - 1) + 1]) row[f] = 0u;
+  }
+}
+
 // ============================ verification ===========================================
 constexpr int kVerifyThreads = 128, kVerifyCtas = 5;  // k_verify: 4 warps per CTA, 5 CTAs per SM (shared memory)
 
@@ -2223,12 +2322,12 @@ __global__ void k_best(const sgtd_candidate *cands, int nq, int k, double icp, s
 // ============================ host driver ================================================
 static float ev_ms(cudaEvent_t a, cudaEvent_t b) { float ms = 0; cudaEventElapsedTime(&ms, a, b); return ms; }
 
-// Region search, automatic formulation: the sparse vote runs when the vote-index entries of the allowed
-// keyframes, summed over the batch, are below this share of (queries x entries on this rank).
+// Region and range search, automatic formulation: the sparse vote runs when the vote-index entries of the
+// allowed keyframes, summed over the batch, are below this share of (queries x entries on this rank).
 constexpr double kRegionSparseShare = 0.0015;
 
 int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, SearchMode mode, int64_t loop_skip) {
-  const bool region = mode == SearchMode::Region, loops = mode == SearchMode::Loops;
+  const bool region = mode == SearchMode::Region, loops = mode == SearchMode::Loops, ranges = mode == SearchMode::Ranges;
   cudaStream_t st = h->stream;
   int rc = finalize_db(h);
   if (rc) return rc;
@@ -2301,8 +2400,8 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, Sea
   size_t o_jd = o; o += run_join ? al((size_t)std::max<int64_t>(qb->n, 1) * sizeof(JoinDesc)) : 0;
   size_t o_pose = o; o += al((size_t)std::max(nq * k, 1) * kMaxHyp * 12 * sizeof(double));
   size_t o_jcub = o; o += al(cubj);
-  // region search: per-query counts and offsets of the allowed keyframes, their entries, scan temp
-  const bool region_votes = region && nq > 0 && F > 0;
+  // region / range search: per-query counts and offsets of the allowed keyframes, their entries, scan temp
+  const bool region_votes = (region || ranges) && nq > 0 && F > 0;
   size_t cubr = 0;
   if (region_votes) cub::DeviceScan::ExclusiveSum(nullptr, cubr, (int64_t *)nullptr, (int64_t *)nullptr, nq + 1, st);
   size_t o_rcnt = o; o += region_votes ? al((size_t)(nq + 1) * 8) : 0;
@@ -2349,18 +2448,21 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, Sea
   SGTD_CUDA(h, cudaMemsetAsync(r->votes.p, 0, (size_t)nq * Fa * 4, st));
   SGTD_CUDA(h, cudaMemsetAsync(r->counters.p, 0, 8 * 8, st));
   SGTD_CUDA(h, cudaEventRecord(ev[7], st));
-  // region search: allowed sets of this rank's keyframes, then the vote formulation.  The sparse one needs
-  // every query in the probe-multimap format (kInvMaxDesc descriptors at most).
+  // region / range search: allowed sets of this rank's keyframes, then the vote formulation.  The sparse one
+  // needs every query in the probe-multimap format (kInvMaxDesc descriptors at most).
   bool sparse = false, tables_ready = false;
   std::vector<int64_t> roff;
   const int64_t npos = std::min<int64_t>(h->n_pos, F);
   int64_t *d_roff = (int64_t *)(S + o_roff);
+  // range search: the call's range_off, then its ranges
+  const int64_t *rq_off = ranges ? h->range_q.p : nullptr, *rq = ranges ? h->range_q.p + nq + 1 : nullptr;
   if (region_votes) {
     int64_t *d_rcnt = (int64_t *)(S + o_rcnt);
     unsigned long long *d_rent = (unsigned long long *)(S + o_rent), ent = 0;
     SGTD_CUDA(h, cudaMemsetAsync(d_rent, 0, 8, st));
     SGTD_CUDA(h, cudaMemsetAsync(d_rcnt + nq, 0, 8, st));
-    k_region_count<<<nq, kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, h->d_frame_off.p, d_rcnt, d_rent);
+    if (ranges) k_ranges_count<<<nq, kRegionThreads, 0, st>>>(rq_off, rq, h->frame_lo(), F, h->d_frame_off.p, d_rcnt, d_rent);
+    else k_region_count<<<nq, kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, h->d_frame_off.p, d_rcnt, d_rent);
     SGTD_LAUNCHED(h);
     SGTD_CUDA(h, cub::DeviceScan::ExclusiveSum(S + o_rcub, cubr, d_rcnt, d_roff, nq + 1, st));
     SGTD_LAUNCHED(h);
@@ -2375,8 +2477,12 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, Sea
   if (sparse) {
     const int64_t nitems = roff[nq];
     SGTD_CUDA(h, h->region_items.reserve((size_t)std::max<int64_t>(nitems, 1), st, false));
-    k_region_fill<<<nq, kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, d_roff, h->region_items.p, qb->d_off.p,
-                                                 (const uint32_t *)(S + o_qpr), r->counters.p);
+    if (ranges)
+      k_ranges_fill<<<nq, kRegionThreads, 0, st>>>(rq_off, rq, h->frame_lo(), F, d_roff, h->region_items.p, qb->d_off.p,
+                                                   (const uint32_t *)(S + o_qpr), r->counters.p);
+    else
+      k_region_fill<<<nq, kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, d_roff, h->region_items.p, qb->d_off.p,
+                                                   (const uint32_t *)(S + o_qpr), r->counters.p);
     SGTD_LAUNCHED(h);
     for (int qb0 = 0; qb0 < nq; qb0 += qt_group) {
       const int gq = std::min(qt_group, nq - qb0);
@@ -2525,10 +2631,11 @@ int search(sgtd_handle *h, const sgtd_desc_batch *qb, sgtd_search_result *r, Sea
       }
     }
     if (region_votes) {
-      // dense formulation of a region search: clear the votes outside each query's region; the matches
-      // are then counted by k_topk over the allowed keyframes (whatever the vote kernel counted is dropped)
-      k_region_mask<<<dim3((unsigned)nq, (unsigned)std::min<int64_t>((F + kRegionThreads - 1) / kRegionThreads, 65535)),
-                      kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, r->votes.p);
+      // dense formulation of a region / range search: clear the votes outside each query's allowed set; the
+      // matches are then counted by k_topk over the allowed keyframes (whatever the vote kernel counted is dropped)
+      const dim3 mgrid((unsigned)nq, (unsigned)std::min<int64_t>((F + kRegionThreads - 1) / kRegionThreads, 65535));
+      if (ranges) k_ranges_mask<<<mgrid, kRegionThreads, 0, st>>>(rq_off, rq, h->frame_lo(), F, r->votes.p);
+      else k_region_mask<<<mgrid, kRegionThreads, 0, st>>>(h->pos.p, npos, F, h->region_q.p, r->votes.p);
       SGTD_LAUNCHED(h);
       SGTD_CUDA(h, cudaGetLastError());
       SGTD_CUDA(h, cudaMemsetAsync(r->counters.p + 4, 0, 8, st));
